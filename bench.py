@@ -2,7 +2,7 @@
 """Benchmark of the SCD naming round (BASELINE.json metric: ms per naming round = one k-means iteration
 + full-vocabulary scoring with per-image top-k + per-cluster vote).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config C2]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config C2] [--dump-outputs DIR]
 
 * default arm: the B200 path.  `value` = ms per round of the HEADLINE config (C2, the 1-GPU configuration the metric is
   quoted on) with all inputs resident in HBM (CUDA events, max over ranks, rounds replayed as CUDA graphs); `e2e` = the same
@@ -144,19 +144,48 @@ def sha(t: torch.Tensor) -> str:
     return hashlib.sha1(t.detach().contiguous().cpu().numpy().tobytes()).hexdigest()[:16]
 
 
+DUMP_BYTES = 60 << 20              # array data of --dump-outputs: with the .npy headers the files stay under 64 MB
+PER_ROW_OUTPUTS = ('labels', 'topk_vals', 'topk_idx')
+
+
+def dump_outputs(out_dir, outputs, n_rows):
+    """Writes `outputs` (Round.outputs) as `out_dir/<name>.npy`, so that two builds run with the same arguments can be
+    compared array by array: float32 results stay float32, everything else becomes float64, which holds every integer
+    result exactly.  If the per-row arrays would take the total past DUMP_BYTES, the same rows are kept of each: a
+    sample drawn with a fixed seed, whose row numbers are written as row_index.npy."""
+    arrays = {k: a.astype(np.float32 if a.dtype == np.float32 else np.float64) for k, a in outputs.items()}
+    fixed = sum(a.nbytes for k, a in arrays.items() if k not in PER_ROW_OUTPUTS)
+    row_bytes = sum(arrays[k].nbytes for k in PER_ROW_OUTPUTS) // n_rows
+    if fixed + row_bytes * n_rows > DUMP_BYTES:
+        keep = (DUMP_BYTES - fixed) // (row_bytes + 8)
+        if keep < 1:
+            raise ValueError(f'--dump-outputs: the per-cluster arrays alone take {fixed} bytes, over the {DUMP_BYTES}-byte limit')
+        rows =np.sort(np.random.default_rng(0).choice(n_rows, keep, replace=False))
+        arrays.update({k: arrays[k][rows] for k in PER_ROW_OUTPUTS}, row_index=rows.astype(np.float64))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + '.npy'), a)
+
+
 # ------------------------------------------------------------------------------------------ CPU legs
 _CPU_DATA = {}
 _REF_PD = []
 
 
+def reference_dir():
+    """The checkout of the reference project named by SCD_REFERENCE_DIR, or None (it is not part of this repository)."""
+    ref = os.environ.get('SCD_REFERENCE_DIR', '')
+    return ref if ref and os.path.isdir(os.path.join(ref, 'local_utils')) else None
+
+
 def reference_pairwise_distance():
     """The reference's own `pairwise_distance` (local_utils/faster_mix_k_means_pytorch.py:177), imported unmodified when
-    the checkout is present (the build container); None on the GPU box, where the CPU legs run the oracle port.  The
-    inline naming / vote blocks of main_*.py are script code and are always the oracle's restatement."""
+    SCD_REFERENCE_DIR names a checkout; None otherwise, and the CPU legs run the oracle port.  The inline naming / vote
+    blocks of main_*.py are script code and are always the oracle's restatement."""
     if not _REF_PD:
         fn = None
-        ref = os.environ.get('SCD_REFERENCE_DIR', '/root/reference')
-        if os.path.isdir(os.path.join(ref, 'local_utils')):
+        ref = reference_dir()
+        if ref is not None:
             try:
                 import importlib.util
                 spec = importlib.util.spec_from_file_location('_scd_ref_kmeans', os.path.join(ref, 'local_utils', 'faster_mix_k_means_pytorch.py'))
@@ -316,8 +345,11 @@ class Round:
     against its vocabulary-column shard, the partial [rows, k] lists are all-gathered inside the group and merged by
     the k-way merge kernel (vocab_ways = world: every rank scores all rows, BASELINE.json configs[3]).
 
-    Successive rounds are successive k-means iterations: the centres ping-pong between two buffers and
-    scd_finalize_centers leaves the next E-step's operands in place, exactly like K_Means._lloyd."""
+    Every round is one k-means iteration from the initial centroids C0, so its inputs, and with them its results, are
+    the same from round to round and from run to run (the fp32 M-step sums vary in their last bits from run to run;
+    iterated, that would change labels).  The round still does the work of an iteration of K_Means._lloyd:
+    scd_finalize_centers leaves the new centres' E-step operands in `estep_next`, while the planes of C0 stay in
+    `estep`."""
 
     def __init__(self, cfg, rank, world, group, naming_shard='rows', vocab_ways=None, data=None, host_data=None, exchange='peer',
                  fused_em=False):
@@ -335,11 +367,11 @@ class Round:
         own = lambda t: t.clone() if t.is_cuda else t.to(dev).contiguous()       # never keep a view of the whole config alive
         self.X = own(data['X'][self.row_lo:self.row_hi])
         self.C0 = data['C0'].to(dev).contiguous()
-        self.C = [self.C0.clone(), torch.empty_like(self.C0)]
-        self.cur = 0
+        self.centers = torch.empty_like(self.C0)
         self.inertia = torch.zeros(1, dtype=torch.float64, device=dev)
         self.mstep = kmeans._MStep(n_local, d, cfg.k, dev)
         self.estep = kmeans._EStep(cfg.k, d, dev)
+        self.estep_next = kmeans._EStep(cfg.k, d, dev)
         self.fused_em = fused_em and self.estep.fusable(n_local)
         self.km = kmeans.K_Means(k=cfg.k, process_group=group if world > 1 else None)
         self.labels = torch.empty(n_local, dtype=torch.int64, device=dev)
@@ -404,7 +436,7 @@ class Round:
         launches = 0
         mark = (lambda i: ev_phase[i].record()) if ev_phase is not None else (lambda i: None)
         mark(0)
-        c_old, c_new = self.C[self.cur], self.C[self.cur ^ 1]
+        c_old, c_new = self.C0, self.centers
         # ---- k-means iteration: E-step, M-step sums, (all-reduce), divide (+ next E-step's operands)
         inertia = self.inertia
         if self.px is not None:                     # this round's [sums | counts | inertia] block, mapped by every rank
@@ -419,13 +451,14 @@ class Round:
             self.estep.run(self.X, c_old, self.labels, inertia); launches += 1 if ready else 2     # (centroid split +) E-step
             mark(1)
             self.mstep.sums_counts(self.X, self.labels); launches += 3                # hist+scan, scatter, segment sum
+        self.estep.ready_for = c_old.data_ptr()     # the planes of C0 stay in `estep`: the next round starts from C0 too
         mark(2)
         if self.px is not None:                     # all-reduce over peer loads + divide + next E-step operands: one launch
-            self.mstep.finalize_peer(c_old, c_new, self.inertia_red, estep=self.estep); launches += 1
+            self.mstep.finalize_peer(c_old, c_new, self.inertia_red, estep=self.estep_next); launches += 1
         else:
             counts_f = self.km._allreduce(self.mstep, self.inertia)
             launches += 1 if counts_f is not None else 0                              # pack (the all-reduce is NCCL's)
-            self.mstep.finalize(c_old, c_new, counts_f, estep=self.estep, shift=False); launches += 1
+            self.mstep.finalize(c_old, c_new, counts_f, estep=self.estep_next, shift=False); launches += 1
         mark(3)
         # ---- full-vocabulary scoring + per-image top-5
         if ev_name is not None:
@@ -465,30 +498,29 @@ class Round:
             out = nm.vote_records(records, cfg.k, NUM_COMMON, plan=self.vote_plan); launches += 3
             self.records = records
         mark(6)
-        self.cur ^= 1
         self.launches_per_round = launches
         self.last = (vals, idx, out)
         return out
 
-    def reset(self):
-        """Back to the initial centroids (the parity round starts from them on every N)."""
-        self.C[0].copy_(self.C0)
-        self.cur = 0
-        self.estep.ready_for = None
+    def outputs(self):
+        """Host copies of what the last round handed its caller: labels and inertia of the E-step, the new centres,
+        top-k values and indices, and the vote (at N > 1 the per-row arrays are this rank's shard)."""
+        vals, idx, (names, counts, distinct, rows, _) = self.last
+        out = dict(labels=self.labels, inertia=self.inertia, centers=self.centers, topk_vals=vals, topk_idx=idx,
+                   vote_names=names, vote_counts=counts, vote_distinct=distinct, cluster_rows=rows)
+        return {k: t.cpu().numpy() for k, t in out.items()}
 
     def capture(self, n_graphs=2):
-        """Record rounds into CUDA graphs (the round is launch-bound at N > 1).  Successive rounds alternate between the
-        two centre buffers, so graphs come in pairs: graphs[i] is the round that starts from C[i & 1].  Every graph
-        carries its own pair of EXTERNAL timing events around the scoring/top-k launches (event-record nodes), so the
-        dominant kernel is timed inside the replayed, back-to-back region itself - one sample per timed step."""
-        n_graphs = max(2, n_graphs + (n_graphs & 1))
+        """Record rounds into CUDA graphs (the round is launch-bound at N > 1), one per timed step up to `n_graphs`, all
+        of the same round.  Every graph carries its own pair of EXTERNAL timing events around the scoring/top-k launches
+        (event-record nodes), so the dominant kernel is timed inside the replayed, back-to-back region itself - one
+        sample per timed step."""
+        n_graphs = max(1, n_graphs)
         try:
             side = torch.cuda.Stream()
             side.wait_stream(torch.cuda.current_stream())
             with torch.cuda.stream(side):
-                if self.cur != 0:
-                    self.run()
-                self.run(); self.run()                       # steady state: the operands of C[0] are in the E-step workspace
+                self.run(); self.run()                       # steady state: the planes of C0 are in the E-step workspace
             torch.cuda.current_stream().wait_stream(side)
             torch.cuda.synchronize()
             graphs, events, phase_events = [], [], []
@@ -519,8 +551,7 @@ class Round:
         if self.graphs is not None:
             self.graphs[self.gstep % len(self.graphs)].replay()
             self.gstep += 1
-            self.cur ^= 1
-            self.estep.ready_for = self.C[self.cur].data_ptr()
+            self.estep.ready_for = self.C0.data_ptr()
         else:
             self.run()
 
@@ -555,9 +586,10 @@ class Round:
         self.graphs = None
 
 
-def measure(rnd, steps, warmup, world, group, use_graph, sampler=None):
+def measure(rnd, steps, warmup, world, group, use_graph, sampler=None, keep_outputs=False):
     """Warm up, (capture,) time `steps` rounds with CUDA events between barriers, then time the scoring/top-k launches
-    of a few eager rounds.  Returns (ms_per_step, naming_ms, graphed) as the max over ranks."""
+    of a few eager rounds.  Returns (ms_per_step, naming_ms, graphed) as the max over ranks.  `keep_outputs`: host
+    copies of the last timed round's results go to `rnd.timed_outputs`, taken before any later round overwrites them."""
     def barrier():
         if world > 1:
             import torch.distributed as dist
@@ -594,6 +626,8 @@ def measure(rnd, steps, warmup, world, group, use_graph, sampler=None):
     ev1.record()
     barrier()
     ms_total = ev0.elapsed_time(ev1)
+    if keep_outputs:
+        rnd.timed_outputs = rnd.outputs()
     # the dominant kernel, timed live INSIDE the timed region: event-record nodes of the replayed graphs (or the eager
     # events above); only if a graph could not carry events, a few eager rounds right after the region
     per_step = rnd.graph_kernel_ms(steps) if graphed else [a.elapsed_time(b) for a, b in name_evs]
@@ -623,7 +657,6 @@ def parity_block(rnd, data, world, group):
     values a reader compares the N > 1 lines with."""
     from scd_b200 import kmeans, naming
     cfg = rnd.cfg
-    rnd.reset()
     names, counts, _, _, ovf = rnd.run()
     vals, idx, _ = rnd.last
     torch.cuda.synchronize()
@@ -749,6 +782,8 @@ def main():
     ap.add_argument('--no-clocks', action='store_true')
     ap.add_argument('--no-extra', action='store_true', help='skip the c5 / c4_vocab_shard / sustained blocks')
     ap.add_argument('--extra-steps', type=int, default=5)
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the results of the last timed round as DIR/<name>.npy (one GPU, B200 arm; at most 64 MB)')
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == 'b200' else args.warmup
 
@@ -757,6 +792,8 @@ def main():
     rank = int(os.environ.get('RANK', '0'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
+    if args.dump_outputs and (args.impl != 'b200' or world > 1):
+        ap.error('--dump-outputs writes the round of the B200 arm in one process: use it with --impl b200 and no launcher')
     feat_mb = cfg.n * synth.D * 6 / 1e6
     voc_mb = cfg.v * synth.D * 2 / 1e6
     if world == 1:
@@ -795,7 +832,7 @@ def main():
                               warmup=args.warmup, ms_per_step=round(v, 1), higher_is_better=False, scaling='strong',
                               vs_baseline=None, dtype='f32', data='synthetic', config=config,
                               cpu_baseline=dict(value=round(v, 1), unit='ms', cores=threads, kind=cpu_kind(), kind_detail=CPU_KIND_DETAIL[cpu_kind()], sample=sample, split_ms=detail,
-                                                reference_checkout_present=os.path.isdir('/root/reference')),
+                                                reference_checkout_present=reference_dir() is not None),
                               e2e=dict(value=round(v, 1), unit='ms', h2d_bytes_per_step=0, d2h_bytes_per_step=0))))
         return 0
 
@@ -817,8 +854,11 @@ def main():
     rnd = Round(cfg, rank, world, group, args.naming_shard, args.vocab_ways or None, host_data=host, exchange=args.exchange, fused_em=args.fused_em)
 
     sampler = ClockSampler(physical_gpu_index(local_rank), enabled=not args.no_clocks)
-    ms_per_step, name_ms, graphed = measure(rnd, args.steps, args.warmup, world, group, not args.no_graph, sampler)
+    ms_per_step, name_ms, graphed = measure(rnd, args.steps, args.warmup, world, group, not args.no_graph, sampler,
+                                            keep_outputs=bool(args.dump_outputs))
     clocks = sampler.result()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, rnd.timed_outputs, cfg.n)
     launches_per_round = rnd.launches_per_round
     phase_us = getattr(rnd, 'phase_us', None)
     fused_flag = rnd.fused_em
@@ -900,7 +940,7 @@ def main():
         threads = os.cpu_count() or 1
         v, detail, n_s = cpu_round_ms(cfg, CPU_SAMPLE_ROWS, threads, repeats=2)
         cpu_baseline = dict(value=round(v, 1), unit='ms', cores=threads, kind=cpu_kind(), kind_detail=CPU_KIND_DETAIL[cpu_kind()], split_ms=detail,
-                            reference_checkout_present=os.path.isdir('/root/reference'),
+                            reference_checkout_present=reference_dir() is not None,
                             sample=f'{n_s} of {cfg.n} rows (all {cfg.k} centroids, all {cfg.v} names), time scaled linearly in rows')
 
     # the other BASELINE.json configs on the same N GPUs

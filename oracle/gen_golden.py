@@ -1,9 +1,14 @@
 #!/usr/bin/env python
 """Generate ``tests/golden/*.npz`` by running the REAL reference code on seeded inputs.
 
-TEST INFRASTRUCTURE.  Runs only where the reference checkout exists (the build container,
-``/root/reference``); the fixtures it writes are committed so that nothing on the GPU box ever
-needs the checkout.  Re-run with:  ``python -m oracle.gen_golden [--ref /root/reference]``.
+TEST INFRASTRUCTURE.  Runs only with a checkout of the reference project (not part of this repository);
+the fixtures it writes are committed so that the tests never need the checkout.  Re-run with:
+``PYTHONHASHSEED=0 python -m oracle.gen_golden --ref <checkout>`` (or SCD_REFERENCE_DIR=<checkout>).
+
+``naming_ptsup_strings.npz`` was first written without a checkout, by ``oracle.naming_oracle.naming_loop_ptsup``, the
+restatement that the live comparison in tests/test_golden_reproducible_cpu.py matched against the reference's loop
+text; regenerating it from a checkout (``--only naming_strings``) replaces it with the reference's own trace, and that
+test compares the two bit for bit.
 
 What is executed from the reference (never copied into this repo):
   * imported as modules: ``local_utils/faster_mix_k_means_pytorch.py`` (K_Means, pairwise_distance),
@@ -342,6 +347,77 @@ def gen_naming(ref, lang):
     np.savez_compressed(os.path.join(OUT, 'naming_small.npz'), **res)
 
 
+PTSUP_STRINGS_HASH_SEED = '0'
+
+
+def ptsup_strings_case():
+    """Inputs of the partially supervised voting loop with STRING names: the vocabulary is not in lexicographic order and
+    holds duplicate names (``sorted(cand_names)`` main_ptsup.py:659 sorts strings, ``nouns.index`` resolves a duplicate to
+    its first column).  The loop's ``list(set(...) - set(...))`` order depends on string hashing, so a trace of it is only
+    reproducible under a fixed PYTHONHASHSEED (PTSUP_STRINGS_HASH_SEED)."""
+    d, v, k_true, n = 32, 300, 10, 2500
+    g = torch.Generator().manual_seed(21)
+    W = bf16_round(unit_rows(torch.randn(v, d, generator=g))).t().contiguous()
+    feats, y = clustered_feats(n, d, k_true, seed=100 + n)
+    feats = bf16_round(feats)
+    idx_top = (100. * feats @ W).topk(5, 1, True, True)[1]
+    rs = np.random.RandomState(3)
+    nouns = ['n%05d' % x for x in rs.permutation(v)]                  # column order != lexicographic order
+    for a, b in ((7, 150), (20, 21), (40, 299)):                      # duplicate names: nouns.index -> first column
+        nouns[b] = nouns[a]
+    g2 = torch.Generator().manual_seed(5)
+    noise = torch.randint(0, k_true, (n,), generator=g2)
+    flip = torch.rand(n, generator=g2) < 0.15
+    preds0 = torch.where(flip, noise, y).numpy().astype(np.int64)
+    mask_lab = ((y < k_true // 2) & (torch.rand(n, generator=torch.Generator().manual_seed(6)) < 0.5)).numpy()
+    all_preds = preds0.copy()
+    all_preds[mask_lab] = y.numpy()[mask_lab]
+    lab_idx = [int(idx_top[(y == c).numpy() & mask_lab][:, 0].mode().values) for c in range(k_true // 2)]
+    lab_idx = list(dict.fromkeys(lab_idx))
+    lab_names = list(dict.fromkeys(nouns[i] for i in lab_idx))
+    lab_idx = [nouns.index(s) for s in lab_names]
+    return dict(W=W, feats=feats, idx_top=idx_top, nouns=nouns, all_preds=all_preds, mask_lab=mask_lab, lab_idx=lab_idx,
+                lab_names=lab_names, k_true=k_true)
+
+
+def run_reference_ptsup_strings(ref, lang, c):
+    """The reference's own loop text (main_ptsup.py) on ``ptsup_strings_case()``: per round (voted names, candidate
+    names, u_preds, number of distinct voted names)."""
+    loop_ptsup, _ = source_block(os.path.join(ref, 'main_ptsup.py'), 'while (set(cur_voted_names)', 'u_preds = logits.argmax')
+    mask_lab, all_preds, nouns, k_true = c['mask_lab'], c['all_preds'], c['nouns'], c['k_true']
+    u_preds, l_preds = all_preds[~mask_lab], all_preds[mask_lab]
+    args = _Args()
+    args.num_common_vote, args.num_common_linear, args.n_cluster, args.dataset_name = 20, 4, k_true, 'cub'
+    trace = []
+    ns = dict(args=args, name_idx_top5=c['idx_top'][~mask_lab], u_preds=u_preds.copy(), nouns=nouns,
+              zeroshot_weights=c['W'], clip_u_feats=c['feats'][~mask_lab], lab_names=c['lab_names'],
+              num_unlab_classes=k_true - len(c['lab_names']), known_name_idx=[nouns.index(x) for x in c['lab_names']],
+              unlab_cluster_idx=list(set(list(set(all_preds))) - set(list(set(l_preds)))),
+              cur_voted_names=[0.5], prev_voted_names=[1.5], top_k=5, it=0, Counter=Counter, copy=copy,
+              torch=torch, assign_name=lang.assign_name, print=lambda *a, **k: None,
+              _rec=lambda names, cand, p, nu: trace.append((list(names), list(cand), np.array(p).copy(), nu)))
+    body = loop_ptsup.replace('u_preds = logits.argmax(dim=-1).view(-1).cpu().numpy()',
+                              'u_preds = logits.argmax(dim=-1).view(-1).cpu().numpy()\n'
+                              '    _rec(cur_voted_names, cand_names, u_preds, len(voted_unique_name_idx))')
+    exec(body, ns)
+    return trace
+
+
+def save_ptsup_strings_trace(path, trace):
+    out = dict(rounds=np.int64(len(trace)), hash_seed=np.array(PTSUP_STRINGS_HASH_SEED))
+    for r, (names, cand, p, nu) in enumerate(trace):
+        out.update({f'voted_{r}': np.array(names, dtype=str), f'cand_{r}': np.array(cand, dtype=str),
+                    f'preds_{r}': np.asarray(p, dtype=np.int64), f'nuniq_{r}': np.int64(nu)})
+    np.savez_compressed(path, **out)
+
+
+def gen_naming_strings(ref, lang):
+    if os.environ.get('PYTHONHASHSEED') != PTSUP_STRINGS_HASH_SEED:
+        raise SystemExit(f'naming_strings: run with PYTHONHASHSEED={PTSUP_STRINGS_HASH_SEED} (the loop iterates string sets)')
+    save_ptsup_strings_trace(os.path.join(OUT, 'naming_ptsup_strings.npz'),
+                             run_reference_ptsup_strings(ref, lang, ptsup_strings_case()))
+
+
 # ------------------------------------------------------------------ evaluation + on-disk contract fixtures
 class _FakeImages:
     """Stands in for an image batch: ``extract_feature`` only calls ``.cuda()`` on it and hands it to the model."""
@@ -427,11 +503,13 @@ def gen_eval(ref):
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument('--ref', default='/root/reference')
+    ap.add_argument('--ref', default=os.environ.get('SCD_REFERENCE_DIR'), help='checkout of the reference project')
     ap.add_argument('--out', default=None, help='write the fixtures here instead of tests/golden (used by the reproducibility test)')
-    ap.add_argument('--only', default=None, choices=[None, 'kmeans', 'constrained', 'hungarian', 'naming', 'eval'],
+    ap.add_argument('--only', default=None, choices=[None, 'kmeans', 'constrained', 'hungarian', 'naming', 'naming_strings', 'eval'],
                     help='regenerate one fixture family (the others are left as committed)')
     a = ap.parse_args()
+    if not a.ref:
+        ap.error('--ref (or SCD_REFERENCE_DIR) must name a checkout of the reference project')
     global OUT
     if a.out:
         OUT = os.path.abspath(a.out)
@@ -447,6 +525,8 @@ def main():
         gen_hungarian(cu)
     if todo('naming'):
         gen_naming(a.ref, lang)
+    if todo('naming_strings'):
+        gen_naming_strings(a.ref, lang)
     if todo('eval'):
         gen_eval(a.ref)
     for f in sorted(os.listdir(OUT)):

@@ -1,6 +1,6 @@
-"""CPU only, and only where the reference checkout exists (the build container; skipped on the GPU box): the committed
-fixtures are what the REAL reference code produces today - regenerate every family into a scratch directory with
-oracle/gen_golden.py and compare array by array."""
+"""CPU only, and only with a checkout of the reference project named by SCD_REFERENCE_DIR (it is not part of this
+repository; skipped without it): the committed fixtures are what the REAL reference code produces today - regenerate
+every family into a scratch directory with oracle/gen_golden.py and compare array by array."""
 import os
 import subprocess
 import sys
@@ -9,9 +9,10 @@ import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = '/root/reference'
+REF = os.environ.get('SCD_REFERENCE_DIR', '')
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'local_utils')), reason='reference checkout not present')
+pytestmark = pytest.mark.skipif(not REF or not os.path.isdir(os.path.join(REF, 'local_utils')),
+                                reason='needs a checkout of the reference project (SCD_REFERENCE_DIR)')
 
 
 @pytest.mark.parametrize('family,files', [
@@ -19,11 +20,14 @@ pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'local_utils
     ('constrained', ['kmeans_constrained.npz']),
     ('hungarian', ['hungarian.npz']),
     ('naming', ['naming_small.npz']),
+    ('naming_strings', ['naming_ptsup_strings.npz']),
     ('eval', ['eval_small.npz']),
 ])
 def test_fixture_family_regenerates_bit_identically(tmp_path, golden_dir, family, files):
+    from oracle.gen_golden import PTSUP_STRINGS_HASH_SEED
     r = subprocess.run([sys.executable, '-m', 'oracle.gen_golden', '--ref', REF, '--only', family, '--out', str(tmp_path)],
-                       cwd=ROOT, capture_output=True, text=True, timeout=600)
+                       cwd=ROOT, capture_output=True, text=True, timeout=600,
+                       env=dict(os.environ, PYTHONHASHSEED=PTSUP_STRINGS_HASH_SEED))
     assert r.returncode == 0, r.stderr[-2000:]
     for f in files:
         new, old = np.load(tmp_path / f), np.load(os.path.join(golden_dir, f))
@@ -37,58 +41,19 @@ def test_ptsup_loop_with_string_names_matches_the_reference_loop():
     """ADVICE round 1: `sorted(cand_names)` (main_ptsup.py:659) sorts NAME STRINGS and `nouns.index` resolves duplicates
     to the first column.  The real loop text is exec'd here with a string vocabulary that is NOT in lexicographic order
     and contains duplicate names, in the same interpreter as the oracle (the loop's `list(set(...) - set(...))` order
-    depends on the process's string hashing, so no fixture can hold it) - voted names, candidate lists and the
-    re-assigned clusters must agree round by round."""
-    import copy
-    from collections import Counter
-    import torch
+    depends on the process's string hashing; tests/golden/naming_ptsup_strings.npz holds the trace under a fixed
+    PYTHONHASHSEED) - voted names, candidate lists and the re-assigned clusters must agree round by round."""
     from oracle import gen_golden as gg, naming_oracle
     _, _, lang, _ = gg.import_reference(REF)
-    loop_ptsup, _ = gg.source_block(os.path.join(REF, 'main_ptsup.py'), 'while (set(cur_voted_names)', 'u_preds = logits.argmax')
-    d, v, k_true, n = 32, 300, 10, 2500
-    g = torch.Generator().manual_seed(21)
-    W = gg.bf16_round(gg.unit_rows(torch.randn(v, d, generator=g))).t().contiguous()
-    feats, y = gg.clustered_feats(n, d, k_true, seed=100 + n)
-    feats = gg.bf16_round(feats)
-    idx_top = (100. * feats @ W).topk(5, 1, True, True)[1]
-    rs = np.random.RandomState(3)
-    nouns = ['n%05d' % x for x in rs.permutation(v)]                  # column order != lexicographic order
-    for a, b in ((7, 150), (20, 21), (40, 299)):                      # duplicate names: nouns.index -> first column
-        nouns[b] = nouns[a]
-    g2 = torch.Generator().manual_seed(5)
-    noise = torch.randint(0, k_true, (n,), generator=g2)
-    flip = torch.rand(n, generator=g2) < 0.15
-    preds0 = torch.where(flip, noise, y).numpy().astype(np.int64)
-    mask_lab = ((y < k_true // 2) & (torch.rand(n, generator=torch.Generator().manual_seed(6)) < 0.5)).numpy()
-    all_preds = preds0.copy()
-    all_preds[mask_lab] = y.numpy()[mask_lab]
-    lab_idx = [int(idx_top[(y == c).numpy() & mask_lab][:, 0].mode().values) for c in range(k_true // 2)]
-    lab_idx = list(dict.fromkeys(lab_idx))
-    lab_names = list(dict.fromkeys(nouns[i] for i in lab_idx))
-    lab_idx = [nouns.index(s) for s in lab_names]
-    u_preds, l_preds = all_preds[~mask_lab], all_preds[mask_lab]
-
-    class _Args:
-        pass
-    args = _Args()
-    args.num_common_vote, args.num_common_linear, args.n_cluster, args.dataset_name = 20, 4, k_true, 'cub'
-    trace = []
-    ns = dict(args=args, name_idx_top5=idx_top[~mask_lab], u_preds=u_preds.copy(), nouns=nouns,
-              zeroshot_weights=W, clip_u_feats=feats[~mask_lab], lab_names=lab_names,
-              num_unlab_classes=k_true - len(lab_names), known_name_idx=[nouns.index(x) for x in lab_names],
-              unlab_cluster_idx=list(set(list(set(all_preds))) - set(list(set(l_preds)))),
-              cur_voted_names=[0.5], prev_voted_names=[1.5], top_k=5, it=0, Counter=Counter, copy=copy,
-              torch=torch, assign_name=lang.assign_name, print=lambda *a, **k: None,
-              _rec=lambda names, cand, p, nu: trace.append((list(names), list(cand), np.array(p).copy(), nu)))
-    body = loop_ptsup.replace('u_preds = logits.argmax(dim=-1).view(-1).cpu().numpy()',
-                              'u_preds = logits.argmax(dim=-1).view(-1).cpu().numpy()\n'
-                              '    _rec(cur_voted_names, cand_names, u_preds, len(voted_unique_name_idx))')
-    exec(body, ns)
-    got = naming_oracle.naming_loop_ptsup(idx_top[~mask_lab], all_preds.copy(), mask_lab, feats[~mask_lab], W, lab_idx, k_true,
-                                          top_k=5, num_common_vote=20, num_common_linear=4, nouns=nouns)
+    c = gg.ptsup_strings_case()
+    trace = gg.run_reference_ptsup_strings(REF, lang, c)
+    m = c['mask_lab']
+    got = naming_oracle.naming_loop_ptsup(c['idx_top'][~m], c['all_preds'].copy(), m, c['feats'][~m], c['W'], c['lab_idx'],
+                                          c['k_true'], top_k=5, num_common_vote=20, num_common_linear=4, nouns=c['nouns'])
     assert len(trace) >= 2 and len(got) == len(trace)
     for (names, cand, p, nu), r in zip(trace, got):
         assert r['voted'] == names and r['cand'] == cand and r['n_unique'] == nu
         assert np.array_equal(r['u_preds'], p)
     # and the index-named shortcut would NOT have produced this: the lexicographic order differs from the column order
+    nouns = c['nouns']
     assert [nouns.index(s) for s in got[0]['cand']] != sorted(nouns.index(s) for s in got[0]['cand'])

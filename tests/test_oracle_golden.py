@@ -1,6 +1,8 @@
 """The oracle is pinned here: every oracle function is compared with fixtures that were produced by
 running the real reference code (oracle/gen_golden.py).  CPU only."""
 import os
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -159,3 +161,36 @@ def test_eval_oracle_matches_reference(golden_dir):
         assert np.array_equal(np.array(sorted(m.items())), g[f'c{ci}_map'])
         for sub, sel in (('all', np.ones(len(y), bool)), ('old', mask), ('new', ~mask)):
             assert np.array_equal(np.array(eval_oracle.evaluate_semantic_acc(y[sel], names, p[sel], cand)), g[f'c{ci}_sem_{sub}'])
+
+
+_PTSUP_STRINGS = """
+import sys
+from oracle import gen_golden as gg, naming_oracle
+c = gg.ptsup_strings_case()
+m = c['mask_lab']
+got = naming_oracle.naming_loop_ptsup(c['idx_top'][~m], c['all_preds'].copy(), m, c['feats'][~m], c['W'], c['lab_idx'],
+                                      c['k_true'], top_k=5, num_common_vote=20, num_common_linear=4, nouns=c['nouns'])
+gg.save_ptsup_strings_trace(sys.argv[1], [(r['voted'], r['cand'], r['u_preds'], r['n_unique']) for r in got])
+"""
+
+
+def test_ptsup_loop_with_string_names_matches_the_stored_trace(golden_dir, tmp_path):
+    """The partially supervised loop on a string vocabulary that is not in lexicographic order and holds duplicate names
+    (``sorted(cand_names)`` sorts strings, ``nouns.index`` resolves duplicates to the first column), round by round
+    against naming_ptsup_strings.npz.  The loop iterates string sets, so both run under the fixture's PYTHONHASHSEED."""
+    from oracle import gen_golden as gg
+    g = _load(golden_dir, 'naming_ptsup_strings.npz')
+    assert str(g['hash_seed']) == gg.PTSUP_STRINGS_HASH_SEED
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    env = dict(os.environ, PYTHONHASHSEED=gg.PTSUP_STRINGS_HASH_SEED)
+    r = subprocess.run([sys.executable, '-c', _PTSUP_STRINGS, str(tmp_path / 'got.npz')], cwd=root, env=env,
+                       capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stderr[-2000:]
+    got = np.load(tmp_path / 'got.npz')
+    assert int(got['rounds']) == int(g['rounds']) >= 2
+    for k in g.files:
+        assert got[k].dtype == g[k].dtype and np.array_equal(got[k], g[k]), k
+    # the index-named shortcut would NOT have produced this: the lexicographic order differs from the column order
+    nouns = gg.ptsup_strings_case()['nouns']
+    cand = list(g['cand_0'])
+    assert [nouns.index(s) for s in cand] != sorted(nouns.index(s) for s in cand)
