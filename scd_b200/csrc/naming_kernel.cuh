@@ -17,9 +17,10 @@
 // left and the issuer spent 40 % of its time waiting for B (65 % tensor-active).  Now the first TWO 64-wide
 // k-blocks of the rows live in TENSOR MEMORY as the A operand (tcgen05.mma with A from TMEM; loader warps write them
 // with tcgen05.st, thread = row = TMEM lane), the other ten stay in shared memory (SWIZZLE_128B), and the 32 KB
-// that frees plus the old ring hold a 4-deep ring of 112-row x 64-k vocabulary boxes (14 KB per CTA, SWIZZLE_128B).
+// that frees plus the old ring hold a 9-deep ring of 112-row x 32-k vocabulary boxes (7 KB per CTA, SWIZZLE_64B):
+// the two MMAs kk = 0, 1 of a k-block read one stage, kk = 2, 3 the next, so a stage is free again after two MMAs.
 // Wider tiles (224 instead of 192) amortise the fixed per-MMA issue cost over more columns - the tile sweep
-// (96 -> 192 -> 240 -> 224) measured 224 x 2 TMEM k-blocks x 4 stages fastest (2.76 ms on C2).
+// (96 -> 192 -> 240 -> 224) measured 224 x 2 TMEM k-blocks fastest (2.76 ms on C2).
 // TMEM: accumulators at columns [0,224) and [256,480), A k-blocks at [224,256) and [480,512).
 //
 // The epilogue is a two-level selection: per 32-column chunk only the chunk maximum is computed (31 FMNMX) and
@@ -28,12 +29,14 @@
 // exact scan of those k parked chunks at the end of the vocabulary sweep finishes the row.  (The unsupervised
 // driver's softmax additionally keeps a running max / sum-exp.)  Only [N, k] leaves the SM.
 //
-// Warp roles (544 threads): 0, 2 = vocabulary (B) TMA producers (alternate k-blocks; 2 also allocates TMEM),
-// 1, 3, 16 = MMA issuers (leader CTA only, k-blocks round-robin, a shared-memory token keeps the issue order),
-// 4..11 = epilogue (TMEM lane quadrant = warp & 3; warps 4..7 take columns 0..127 of every accumulator tile,
-// warps 8..11 columns 128..223), 12..15 = loaders of the
-// TMEM-resident A k-blocks (global -> registers -> tcgen05.st); 12 is also the TMA producer of the shared-memory
-// A k-blocks.
+// Warp roles (640 threads = 5 warpgroups; setmaxnreg moves registers from the control warps to the epilogue):
+//   WG0 (warps 0..3)   0, 2 = vocabulary (B) TMA producers (2 also allocates TMEM); 1, 3 = MMA issuers
+//   WG1, WG2 (4..11)   epilogue (TMEM lane quadrant = warp & 3; warps 4..7 take columns 0..127 of every accumulator
+//                      tile, warps 8..11 columns 128..223)
+//   WG3 (12..15)       loaders of the TMEM-resident A k-blocks (global -> registers -> tcgen05.st); 12 is also the
+//                      TMA producer of the shared-memory A k-blocks
+//   WG4 (16..19)       16 = third MMA issuer (leader CTA only, k-blocks round-robin, a token keeps the issue order),
+//                      17 = third B producer, 18 and 19 idle
 #pragma once
 #include "ptx.cuh"
 #include <cuda_bf16.h>
@@ -47,13 +50,23 @@ constexpr int kAKBlock = 64;           // k per A / B block  (128 B rows, SWIZZL
 constexpr int kNumAKBlocks = kNameMaxD / kAKBlock;   // 12 (capacity; the live count is NameParams::num_kb)
 constexpr int kTmemAKBlocks = 2;       // A k-blocks 0, 1 live in tensor memory (32 columns above each accumulator)
 constexpr int kSmemAKBlocks = kNumAKBlocks - kTmemAKBlocks;   // 8 in shared memory
-constexpr int kBStages = 4;            // one stage = one k-block (14 KB) of one vocabulary tile
-constexpr int kBProducers = 2;         // warps 0 and 2 issue alternate stages (one warp keeps only one box in flight,
-                                       // ~500-600 cycles each: tools/tma_feed_bench.cu)
+constexpr int kBStageK = 32;           // k per vocabulary stage: half a k-block (64 B rows, SWIZZLE_64B)
+constexpr int kBStages = 9;            // one stage = one 32-k half of a k-block (7 KB) of one vocabulary tile
+constexpr int kBProducers = 3;         // warps 0, 2 and 17 issue stages round-robin (one warp keeps only one box in
+                                       // flight, ~500-600 cycles each: tools/tma_feed_bench.cu); kBStages must be a
+                                       // multiple of it, so that every stage always has the same producer (DESIGN 3.2)
 constexpr int kABlockBytes = kBlockM * kAKBlock * 2;     // 16384
-constexpr int kBStageBytes = (kTileN / 2) * kAKBlock * 2;   // 14336 per CTA
+constexpr int kBStageBytes = (kTileN / 2) * kBStageK * 2;   // 7168 per CTA
 constexpr int kNumIssuers = 3;          // MMA issuer warps 1, 3 and 16, round-robin over k-blocks
-constexpr int kNameThreads = 544;
+constexpr int kNameThreads = 640;
+// per-thread registers after setmaxnreg (launched at 65536 / 640 -> 96): the other warpgroups give up what the
+// epilogue's four 32-column loads in flight need, 2 x (96 - 48) + (96 - 48) = 2 x (168 - 96).  The smallest counts
+// at which ptxas compiles every role of name_topk_kernel<1>, <5> and <8> without spilling.
+constexpr int kCtrlRegs = 48;           // WG0, WG4: producers and issuers
+constexpr int kLoaderRegs = 48;         // WG3: one 32-register row buffer per thread
+constexpr int kEpiRegs = 168;           // WG1, WG2
+static_assert((2 * kCtrlRegs + kLoaderRegs + 2 * kEpiRegs) * 128 <= kNameThreads * 96, "setmaxnreg budget exceeds the launch allocation");
+static_assert(kBStages % kBProducers == 0 && kAKBlock == 2 * kBStageK, "vocabulary ring plan");
 constexpr int kEpiHalves = 2;           // column halves of a tile, one epilogue warp set each
 constexpr int kHalfCols = 128;          // epilogue warps 4..7 take columns [0,128), warps 8..11 columns [128,224)
 constexpr int kTmemCols = 512;
@@ -67,7 +80,7 @@ struct NameSmem {
   // offsets inside dynamic shared memory (base aligned to 1024)
   static constexpr int a_off = 0;
   static constexpr int b_off = kSmemAKBlocks * kABlockBytes;                // 163840
-  static constexpr int bar_off = b_off + kBStages * kBStageBytes;           // 221184
+  static constexpr int bar_off = b_off + kBStages * kBStageBytes;           // 228352
   // barriers (8 B each)
   static constexpr int full_bar = bar_off;                                  // [kBStages]
   static constexpr int empty_bar = full_bar + 8 * kBStages;                 // [kBStages]
@@ -258,42 +271,179 @@ name_topk_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
     return it.t0 + tt;
   };
 
-  if (warp == 0 || warp == 2) {
-    // ======================================================= vocabulary (B) TMA producers
-    // Stage g (a running count over the whole kernel) belongs to producer g % 2.  Whole warp runs the loop
-    // (warp-uniform control flow keeps addresses in uniform registers); one elected lane issues.
-    const uint32_t me = warp == 0 ? 0u : 1u;
-    uint32_t g = 0;
-    const bool prof = p.prof != nullptr;
-    long long pf_t0 = prof ? clock64() : 0, pf_e = 0;
-    for (int l = l_lo; l < l_hi;) {
-      const NameItem it = name_item_at(work, pair, l, l_hi);
-      l += it.nt;
-      const int nt = it.nt;
-      for (int t = 0; t < nt; ++t) {
-        const int v0 = item_tile(it, t) * kTileN + (int)cta_rank * (kTileN / 2);
-        for (int kb = 0; kb < nkb; ++kb, ++g) {
-          if ((g % kBProducers) != me) continue;
-          const int stage = (int)(g % kBStages);
-          const uint32_t phase = (g / kBStages) & 1u;
-          { const long long c0 = prof ? clock64() : 0;
-            ptx::mbar_wait(empty_bar(stage), phase ^ 1, 200 + stage);
-            if (prof) pf_e += clock64() - c0; }
-          if (ptx::elect_one()) {
-            if (leader) ptx::mbar_arrive_expect_tx(full_bar(stage), 2 * kBStageBytes);
-            ptx::tma_load_2d<2>(sbase + NameSmem::b_off + stage * kBStageBytes, &map_w,
-                                full_bar(stage) & ptx::kPeerBitMask, kb * kAKBlock, v0, ptx::kEvictLast);
+  // Registers by role (setmaxnreg acts on whole warpgroups): the epilogue keeps a tile's four 32-column loads in
+  // flight (128 registers of scores); producers and issuers live on uniform registers, a loader on one 32-register
+  // row buffer.  Each role's code is dominated by its own setmaxnreg, so ptxas allocates it within that budget.
+  // Every branch ends in its own copy of the teardown: no code is shared after the roles split, which is what lets
+  // ptxas compile each role at its own register count.
+  // Teardown: nobody may free TMEM / exit while the peer can still touch this CTA's memory.
+  auto teardown = [&]() {
+    ptx::tc_fence_before_sync();
+    ptx::cluster_sync_all();
+    if (warp == 2) ptx::tmem_dealloc<2>(tmem_base, kTmemCols);
+  };
+  const uint32_t wg = warp >> 2;
+  if (wg == 0 || wg == 4) {
+    ptx::setmaxnreg_dec<kCtrlRegs>();
+    if (warp == 0 || warp == 2 || warp == 17) {
+      // ======================================================= vocabulary (B) TMA producers
+      // Stage g (a running count of 32-k halves of k-blocks over the whole kernel) belongs to producer g % 3.  Whole
+      // warp runs the loop (warp-uniform control flow keeps addresses in uniform registers); one elected lane issues.
+      // A half that lies wholly beyond D (ragged last k-block) is still loaded: TMA fills it with zeros.
+      const uint32_t me = warp == 0 ? 0u : (warp == 2 ? 1u : 2u);
+      uint32_t g = 0;
+      const bool prof = p.prof != nullptr;
+      long long pf_t0 = prof ? clock64() : 0, pf_e = 0;
+      for (int l = l_lo; l < l_hi;) {
+        const NameItem it = name_item_at(work, pair, l, l_hi);
+        l += it.nt;
+        const int nt = it.nt;
+        for (int t = 0; t < nt; ++t) {
+          const int v0 = item_tile(it, t) * kTileN + (int)cta_rank * (kTileN / 2);
+          for (int kb = 0; kb < nkb; ++kb) {
+            for (int hh = 0; hh < 2; ++hh, ++g) {
+              if ((g % kBProducers) != me) continue;
+              const int stage = (int)(g % kBStages);
+              const uint32_t phase = (g / kBStages) & 1u;
+              { const long long c0 = prof ? clock64() : 0;
+                ptx::mbar_wait_nocall(empty_bar(stage), phase ^ 1, 200 + stage);
+                if (prof) pf_e += clock64() - c0; }
+              if (ptx::elect_one()) {
+                if (leader) ptx::mbar_arrive_expect_tx(full_bar(stage), 2 * kBStageBytes);
+                ptx::tma_load_2d<2>(sbase + NameSmem::b_off + stage * kBStageBytes, &map_w,
+                                    full_bar(stage) & ptx::kPeerBitMask, kb * kAKBlock + hh * kBStageK, v0, ptx::kEvictLast);
+              }
+              __syncwarp();
+            }
           }
-          __syncwarp();
         }
       }
-    }
-    if (prof && lane == 0) {
-      long long* o = p.prof + (size_t)pair * 32;
-      const int base = (leader ? 0 : 16) + 6 + 6 * (int)me;         // leader: 6,7 / 12,13; peer: 22,23 / 28,29
-      o[base] = clock64() - pf_t0; o[base + 1] = pf_e;
-    }
-  } else if (warp >= 12 && warp < 16) {
+      if (prof && lane == 0) {
+        long long* o = p.prof + (size_t)pair * 32;
+        const int base = (leader ? 0 : 16) + (me == 0 ? 6 : (me == 1 ? 12 : 14));   // leader: 6,7 / 12,13 / 14,15; peer: +16
+        o[base] = clock64() - pf_t0; o[base + 1] = pf_e;
+      }
+    } else if (warp == 1 || warp == 3 || warp == 16) {
+      // ======================================================= MMA issuers (leader CTA; one elected lane of each issues)
+      // What the measurements say about issuing (tools/mma_rate_bench.cu, profiles/r1_mma_rate_*.txt): the tensor pipe
+      // runs an MMA in exactly N/2 cycles when the next one is already queued, the queue is only a couple of MMAs deep,
+      // and a tcgen05.mma keeps the uniform registers of its descriptors busy until it has run - so an issuer that
+      // prepares the next k-block's descriptors after its own MMAs does so behind an idle pipe (+43 cycles per MMA).
+      // Two warps therefore take alternate k-blocks (running count g): each has its own uniform registers, computes
+      // its descriptors and does its barrier waits while the other warp's four MMAs run, then waits for a named-barrier
+      // token (ids 1 / 2) and fires its four MMAs back to back.  The token keeps the issue order, which is also the
+      // execution order of the pipe, so the last k-block's commit covers the whole tile.
+      if (leader) {
+        const uint32_t me = warp == 1 ? 0u : (warp == 3 ? 1u : 2u);
+        const uint32_t idesc = ptx::make_idesc_bf16_f32(2 * kBlockM, kTileN);
+        uint32_t g = 0, tile_no = 0;
+        int my_item_no = 0;
+        const long long g_total = (long long)(l_hi - l_lo) * nkb;
+        const bool prof = p.prof != nullptr && me == 0;
+        long long pf_t0 = prof ? clock64() : 0, pf_te = 0, pf_a = 0, pf_b = 0, pf_tok = 0;
+        const uint64_t pf_ns0 = prof ? ptx::globaltimer_stable_ns() : 0;          // wall time of the same span: clock rate
+        long long* const trace = (p.prof != nullptr && pair == 0 && me < 2) ? p.prof + (size_t)n_pairs * 32 + me * 384 : nullptr;
+        int n_ev = 0;
+        for (int l = l_lo; l < l_hi; ++my_item_no) {
+          const NameItem it = name_item_at(work, pair, l, l_hi);
+          l += it.nt;
+          const int nt = it.nt;
+          for (int t = 0; t < nt; ++t, ++tile_no) {
+            const uint32_t buf = tile_no & 1u;
+            const uint32_t d_tmem = tmem_base + buf * kAccStride;
+            for (int kb = 0; kb < nkb; ++kb, ++g) {
+              if ((g % kNumIssuers) != me) continue;
+              // k-block g reads vocabulary stages 2g (MMAs kk = 0, 1) and 2g + 1 (kk = 2, 3)
+              const int stage0 = (int)((2 * g) % kBStages), stage1 = (int)((2 * g + 1) % kBStages);
+              const uint32_t phase0 = ((2 * g) / kBStages) & 1u, phase1 = ((2 * g + 1) / kBStages) & 1u;
+              // operands of the four MMAs, ready in registers before the token arrives
+              const bool a_in_tmem = kb < kTmemAKBlocks;
+              const uint32_t b_addr0 = sbase + NameSmem::b_off + stage0 * kBStageBytes;
+              const uint32_t b_addr1 = sbase + NameSmem::b_off + stage1 * kBStageBytes;
+              const uint32_t a_addr = sbase + NameSmem::a_off + (a_in_tmem ? 0 : kb - kTmemAKBlocks) * kABlockBytes;
+              uint64_t bd[4], ad[4];
+              uint32_t at[4];
+  #pragma unroll
+              for (int kk = 0; kk < 4; ++kk) {
+                bd[kk] = ptx::make_kmajor_desc((kk < 2 ? b_addr0 : b_addr1) + (kk & 1) * 32, 64);
+                ad[kk] = ptx::make_kmajor_desc(a_addr + kk * 32, 128);
+                at[kk] = tmem_base + a_tmem_col(a_in_tmem ? kb : 0, kk);
+                asm volatile("" : "+l"(bd[kk]), "+l"(ad[kk]), "+r"(at[kk]));
+              }
+              // Accumulator buffer free / rows of the item loaded?  Waited for ahead of the token - except when a tile has fewer
+              // k-blocks than there are issuers (D <= 128).  A parity wait is only sound if the waiter cannot be more than one
+              // phase away from the one it asks for.  With one k-block per tile an issuer sits three tiles ahead of the one it
+              // issued last: the release it needs (tile - 2) can still have the previous release (tile - 4) pending, the wait
+              // returned at once, the MMAs overwrote a buffer the epilogue was reading, and the pair deadlocked (round 1).
+              // With two k-blocks per tile and the ONE-TILE work items the linear partition of round 2 produces at range ends,
+              // an issuer meets k-block kb of an item only every third item: its early wait on a_full(kb) could alias with the
+              // fill before last and the MMAs read rows that were still being written (tools/naming_stress.py: 46 wrong
+              // indices in one launch of 19000 x 5000 x 128 out of ~10^4).  After the token every earlier k-block has been
+              // issued by a warp that waited for its own fill / release, so the barrier is at most one phase behind.
+              const bool te_after_token = nkb < kNumIssuers;
+              if (kb == 0 && !te_after_token) { const long long c0 = prof ? clock64() : 0;
+                ptx::mbar_wait_nocall(tmem_empty_bar(buf), ((tile_no >> 1) & 1u) ^ 1u, 300 + buf);
+                if (prof) pf_te += clock64() - c0; }
+              if (t == 0 && !te_after_token) { const long long c0 = prof ? clock64() : 0;
+                ptx::mbar_wait_nocall(a_full_bar(kb), my_item_no & 1, 400 + kb);
+                if (prof) pf_a += clock64() - c0; }
+              { const long long c0 = prof ? clock64() : 0;
+                ptx::mbar_wait_nocall(full_bar(stage0), phase0, 500 + stage0);
+                ptx::mbar_wait_nocall(full_bar(stage1), phase1, 500 + stage1);
+                if (prof) pf_b += clock64() - c0; }
+              ptx::tc_fence_after_sync();
+              const long long tr0 = trace ? clock64() : 0;
+              // token: the previous issuer has issued k-block g - 1
+              if (g > 0) { const long long c0 = prof ? clock64() : 0;
+                ptx::named_bar_sync(1 + me, 64);
+                if (prof) pf_tok += clock64() - c0; }
+              if (te_after_token) {          // same reasoning for the rows of the item: with one k-block per tile the
+                if (kb == 0) ptx::mbar_wait_nocall(tmem_empty_bar(buf), ((tile_no >> 1) & 1u) ^ 1u, 310 + buf);    // issuers
+                if (t == 0) ptx::mbar_wait_nocall(a_full_bar(kb), my_item_no & 1, 410 + kb);    // take turns on a_full(0) too
+                ptx::tc_fence_after_sync();
+              }
+              const long long tr1 = trace ? clock64() : 0;
+              if (p.prof != nullptr && pair == 0 && t == 0 && kb == 0 && lane == 0 && my_item_no < 64)
+                p.prof[(size_t)n_pairs * 32 + 4 * 384 + my_item_no * 6 + 0] = clock64();            // first k-block of the item issued
+              const bool elected = ptx::elect_one();
+              // the first stage is released as soon as its two MMAs have run, the second after the k-block's last MMA
+              if (elected) {
+                if (a_in_tmem) {
+  #pragma unroll
+                  for (int kk = 0; kk < 4; ++kk) {
+                    ptx::umma_bf16_ts<2>(d_tmem, at[kk], bd[kk], idesc, (kb | kk) != 0 ? 1u : 0u);
+                    if (kk == 1) ptx::umma_commit<2>(empty_bar(stage0), 0b11);
+                  }
+                } else {
+  #pragma unroll
+                  for (int kk = 0; kk < 4; ++kk) {
+                    ptx::umma_bf16<2>(d_tmem, ad[kk], bd[kk], idesc, 1u);
+                    if (kk == 1) ptx::umma_commit<2>(empty_bar(stage0), 0b11);
+                  }
+                }
+              }
+              __syncwarp();
+              if ((long long)g + 1 < g_total) ptx::named_bar_arrive(1 + (me + 1) % kNumIssuers, 64);     // hand the token over ...
+              if (elected) {                                                                            // ... then commit
+                ptx::umma_commit<2>(empty_bar(stage1), 0b11);
+                if (t == nt - 1) ptx::umma_commit<2>(a_empty_bar(kb), 0b11);
+                if (kb == nkb - 1) ptx::umma_commit<2>(tmem_full_bar(buf), 0b11);
+              }
+              __syncwarp();
+              if (trace && lane == 0 && n_ev < 128) { trace[3 * n_ev] = tr0; trace[3 * n_ev + 1] = tr1; trace[3 * n_ev + 2] = clock64(); ++n_ev; }
+            }
+          }
+        }
+        if (prof && lane == 0) {
+          long long* o = p.prof + (size_t)pair * 32;
+          o[0] = clock64() - pf_t0; o[1] = pf_te; o[2] = pf_a; o[3] = pf_b; o[4] = pf_tok; o[5] = tile_no;
+          o[17] = (long long)(ptx::globaltimer_stable_ns() - pf_ns0);
+        }
+      }
+    }                                    // warps 18, 19: no role
+    teardown();
+  } else if (wg == 3) {
+    ptx::setmaxnreg_dec<kLoaderRegs>();
     // ======================================================= loaders of the TMEM-resident A k-blocks
     // thread = image row = TMEM lane; one k-block = 64 bf16 = 32 packed columns.  Global loads of a k-block are in
     // flight before the wait for its columns to be released by the previous item's last tile.
@@ -313,7 +463,7 @@ name_topk_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
           if (row < p.n_rows && kb * kAKBlock + q * 8 < p.d) v = __ldg(src + kb * 8 + q);
           r[4 * q] = v.x; r[4 * q + 1] = v.y; r[4 * q + 2] = v.z; r[4 * q + 3] = v.w;
         }
-        ptx::mbar_wait(a_empty_bar(kb), (my_item_no & 1) ^ 1, 150 + kb);
+        ptx::mbar_wait_nocall(a_empty_bar(kb), (my_item_no & 1) ^ 1, 150 + kb);
         ptx::tc_fence_after_sync();
         ptx::tmem_st_32x32(tmem_base + lane_addr + a_tmem_col(kb, 0), r);
         ptx::tmem_st_wait();
@@ -326,7 +476,7 @@ name_topk_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
       if (warp == 12) {
         const int row0 = it.rb * 2 * kBlockM + (int)cta_rank * kBlockM;
         for (int kb = kTmemAKBlocks; kb < nkb; ++kb) {
-          ptx::mbar_wait(a_empty_bar(kb), (my_item_no & 1) ^ 1, 100 + kb);
+          ptx::mbar_wait_nocall(a_empty_bar(kb), (my_item_no & 1) ^ 1, 100 + kb);
           if (ptx::elect_one()) {
             if (leader) ptx::mbar_arrive_expect_tx(a_full_bar(kb), 2 * kABlockBytes);
             ptx::tma_load_2d<2>(sbase + NameSmem::a_off + (kb - kTmemAKBlocks) * kABlockBytes, &map_x,
@@ -338,112 +488,9 @@ name_topk_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
           p.prof[(size_t)n_pairs * 32 + 4 * 384 + my_item_no * 6 + 5] = clock64();                // the item's rows are on their way
       }
     }
-  } else if (warp == 1 || warp == 3 || warp == 16) {
-    // ======================================================= MMA issuers (leader CTA; one elected lane of each issues)
-    // What the measurements say about issuing (tools/mma_rate_bench.cu, profiles/r1_mma_rate_*.txt): the tensor pipe
-    // runs an MMA in exactly N/2 cycles when the next one is already queued, the queue is only a couple of MMAs deep,
-    // and a tcgen05.mma keeps the uniform registers of its descriptors busy until it has run - so an issuer that
-    // prepares the next k-block's descriptors after its own MMAs does so behind an idle pipe (+43 cycles per MMA).
-    // Two warps therefore take alternate k-blocks (running count g): each has its own uniform registers, computes
-    // its descriptors and does its barrier waits while the other warp's four MMAs run, then waits for a named-barrier
-    // token (ids 1 / 2) and fires its four MMAs back to back.  The token keeps the issue order, which is also the
-    // execution order of the pipe, so the last k-block's commit covers the whole tile.
-    if (leader) {
-      const uint32_t me = warp == 1 ? 0u : (warp == 3 ? 1u : 2u);
-      const uint32_t idesc = ptx::make_idesc_bf16_f32(2 * kBlockM, kTileN);
-      uint32_t g = 0, tile_no = 0;
-      int my_item_no = 0;
-      const long long g_total = (long long)(l_hi - l_lo) * nkb;
-      const bool prof = p.prof != nullptr && me == 0;
-      long long pf_t0 = prof ? clock64() : 0, pf_te = 0, pf_a = 0, pf_b = 0, pf_tok = 0;
-      long long* const trace = (p.prof != nullptr && pair == 0 && me < 2) ? p.prof + (size_t)n_pairs * 32 + me * 384 : nullptr;
-      int n_ev = 0;
-      for (int l = l_lo; l < l_hi; ++my_item_no) {
-        const NameItem it = name_item_at(work, pair, l, l_hi);
-        l += it.nt;
-        const int nt = it.nt;
-        for (int t = 0; t < nt; ++t, ++tile_no) {
-          const uint32_t buf = tile_no & 1u;
-          const uint32_t d_tmem = tmem_base + buf * kAccStride;
-          for (int kb = 0; kb < nkb; ++kb, ++g) {
-            if ((g % kNumIssuers) != me) continue;
-            const int stage = (int)(g % kBStages);
-            const uint32_t phase = (g / kBStages) & 1u;
-            // operands of the four MMAs, ready in registers before the token arrives
-            const bool a_in_tmem = kb < kTmemAKBlocks;
-            const uint32_t b_addr = sbase + NameSmem::b_off + stage * kBStageBytes;
-            const uint32_t a_addr = sbase + NameSmem::a_off + (a_in_tmem ? 0 : kb - kTmemAKBlocks) * kABlockBytes;
-            uint64_t bd[4], ad[4];
-            uint32_t at[4];
-#pragma unroll
-            for (int kk = 0; kk < 4; ++kk) {
-              bd[kk] = ptx::make_kmajor_desc(b_addr + kk * 32, 128);
-              ad[kk] = ptx::make_kmajor_desc(a_addr + kk * 32, 128);
-              at[kk] = tmem_base + a_tmem_col(a_in_tmem ? kb : 0, kk);
-              asm volatile("" : "+l"(bd[kk]), "+l"(ad[kk]), "+r"(at[kk]));
-            }
-            // Accumulator buffer free / rows of the item loaded?  Waited for ahead of the token - except when a tile has fewer
-            // k-blocks than there are issuers (D <= 128).  A parity wait is only sound if the waiter cannot be more than one
-            // phase away from the one it asks for.  With one k-block per tile an issuer sits three tiles ahead of the one it
-            // issued last: the release it needs (tile - 2) can still have the previous release (tile - 4) pending, the wait
-            // returned at once, the MMAs overwrote a buffer the epilogue was reading, and the pair deadlocked (round 1).
-            // With two k-blocks per tile and the ONE-TILE work items the linear partition of round 2 produces at range ends,
-            // an issuer meets k-block kb of an item only every third item: its early wait on a_full(kb) could alias with the
-            // fill before last and the MMAs read rows that were still being written (tools/naming_stress.py: 46 wrong
-            // indices in one launch of 19000 x 5000 x 128 out of ~10^4).  After the token every earlier k-block has been
-            // issued by a warp that waited for its own fill / release, so the barrier is at most one phase behind.
-            const bool te_after_token = nkb < kNumIssuers;
-            if (kb == 0 && !te_after_token) { const long long c0 = prof ? clock64() : 0;
-              ptx::mbar_wait(tmem_empty_bar(buf), ((tile_no >> 1) & 1u) ^ 1u, 300 + buf);
-              if (prof) pf_te += clock64() - c0; }
-            if (t == 0 && !te_after_token) { const long long c0 = prof ? clock64() : 0;
-              ptx::mbar_wait(a_full_bar(kb), my_item_no & 1, 400 + kb);
-              if (prof) pf_a += clock64() - c0; }
-            { const long long c0 = prof ? clock64() : 0;
-              ptx::mbar_wait(full_bar(stage), phase, 500 + stage);
-              if (prof) pf_b += clock64() - c0; }
-            ptx::tc_fence_after_sync();
-            const long long tr0 = trace ? clock64() : 0;
-            // token: the previous issuer has issued k-block g - 1
-            if (g > 0) { const long long c0 = prof ? clock64() : 0;
-              ptx::named_bar_sync(1 + me, 64);
-              if (prof) pf_tok += clock64() - c0; }
-            if (te_after_token) {          // same reasoning for the rows of the item: with one k-block per tile the
-              if (kb == 0) ptx::mbar_wait(tmem_empty_bar(buf), ((tile_no >> 1) & 1u) ^ 1u, 310 + buf);    // issuers
-              if (t == 0) ptx::mbar_wait(a_full_bar(kb), my_item_no & 1, 410 + kb);    // take turns on a_full(0) too
-              ptx::tc_fence_after_sync();
-            }
-            const long long tr1 = trace ? clock64() : 0;
-            if (p.prof != nullptr && pair == 0 && t == 0 && kb == 0 && lane == 0 && my_item_no < 64)
-              p.prof[(size_t)n_pairs * 32 + 4 * 384 + my_item_no * 6 + 0] = clock64();            // first k-block of the item issued
-            const bool elected = ptx::elect_one();
-            if (elected) {
-              if (a_in_tmem) {
-#pragma unroll
-                for (int kk = 0; kk < 4; ++kk) ptx::umma_bf16_ts<2>(d_tmem, at[kk], bd[kk], idesc, (kb | kk) != 0 ? 1u : 0u);
-              } else {
-#pragma unroll
-                for (int kk = 0; kk < 4; ++kk) ptx::umma_bf16<2>(d_tmem, ad[kk], bd[kk], idesc, 1u);
-              }
-            }
-            __syncwarp();
-            if ((long long)g + 1 < g_total) ptx::named_bar_arrive(1 + (me + 1) % kNumIssuers, 64);     // hand the token over ...
-            if (elected) {                                                                            // ... then commit
-              ptx::umma_commit<2>(empty_bar(stage), 0b11);
-              if (t == nt - 1) ptx::umma_commit<2>(a_empty_bar(kb), 0b11);
-              if (kb == nkb - 1) ptx::umma_commit<2>(tmem_full_bar(buf), 0b11);
-            }
-            __syncwarp();
-            if (trace && lane == 0 && n_ev < 128) { trace[3 * n_ev] = tr0; trace[3 * n_ev + 1] = tr1; trace[3 * n_ev + 2] = clock64(); ++n_ev; }
-          }
-        }
-      }
-      if (prof && lane == 0) {
-        long long* o = p.prof + (size_t)pair * 32;
-        o[0] = clock64() - pf_t0; o[1] = pf_te; o[2] = pf_a; o[3] = pf_b; o[4] = pf_tok; o[5] = tile_no;
-      }
-    }
-  } else if (warp >= 4 && warp < 12) {
+    teardown();
+  } else {
+    ptx::setmaxnreg_inc<kEpiRegs>();
     // ======================================================= epilogue: one thread per image row
     const uint32_t quad = warp & 3u;                 // TMEM lane quadrant this warp may read
     const uint32_t half = (warp - 4u) >> 2;          // column half of every tile this warp scans
@@ -505,7 +552,7 @@ name_topk_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
         const int half_cols = half == 0 ? kHalfCols : kTileN - kHalfCols;
         const int n_valid = (int)min((long long)half_cols, p.v_total - col0);      // may be <= 0 on the last tile
         { const long long c0 = prof ? clock64() : 0;
-          ptx::mbar_wait(tmem_full_bar(buf), (tile_no >> 1) & 1u, 600 + buf);
+          ptx::mbar_wait_nocall(tmem_full_bar(buf), (tile_no >> 1) & 1u, 600 + buf);
           if (prof) pf_w += clock64() - c0; }
         ptx::tc_fence_after_sync();
         if (itrace && t == 0) itrace[1] = clock64();                                            // first tile of the item seen
@@ -513,25 +560,26 @@ name_topk_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
         const uint32_t taddr = tmem_base + lane_addr + buf * kAccStride + half * kHalfCols;
         // four 32-column chunks in the first half, three in the second (96 columns).  Its fourth chunk would be the
         // TMEM-resident A columns: never read tensor memory that may not have been written (for D <= 64 the second
-        // A k-block does not exist) - see the E-step epilogue for what that costs
-        uint32_t ra[32], rb[32];
-        ptx::tmem_ld_32x32(taddr, ra);
-        ptx::tmem_ld_wait(ra);                                   // ra = chunk 0
-        ptx::tmem_ld_32x32(taddr + 32, rb);                      // in flight while ra is processed
-        process(ra, col0, n_valid);
-        ptx::tmem_ld_wait(rb);                                   // rb = chunk 1
-        ptx::tmem_ld_32x32(taddr + 64, ra);
-        process(rb, col0 + 32, n_valid - 32);
-        ptx::tmem_ld_wait(ra);                                   // ra = chunk 2
-        if (half == 0) ptx::tmem_ld_32x32(taddr + 96, rb);
-        process(ra, col0 + 64, n_valid - 64);
-        if (half == 0) ptx::tmem_ld_wait(rb);                    // rb = chunk 3
-        // this warp's share of the accumulator buffer is in registers: hand it back to the MMA issuer
+        // A k-block does not exist) - see the E-step epilogue for what that costs.
+        // Every load of the warp's share is in flight before the one wait, and the buffer goes back to the MMA issuer
+        // before any chunk is processed: it is free again one TMEM load latency after the tile completed.
+        uint32_t c0[32], c1[32], c2[32], c3[32];
+        ptx::tmem_ld_32x32(taddr, c0);
+        ptx::tmem_ld_32x32(taddr + 32, c1);
+        ptx::tmem_ld_32x32(taddr + 64, c2);
+        if (half == 0) ptx::tmem_ld_32x32(taddr + 96, c3);
+        ptx::tmem_ld_wait(c0);
+        ptx::tmem_ld_keep(c1);
+        ptx::tmem_ld_keep(c2);
+        if (half == 0) ptx::tmem_ld_keep(c3);
         ptx::tc_fence_before_sync();
         __syncwarp();
         if (lane == 0) ptx::mbar_arrive_remote(tmem_empty_bar(buf) & ptx::kPeerBitMask);
         const long long tr1 = trace ? clock64() : 0;
-        if (half == 0) process(rb, col0 + 96, n_valid - 96);
+        process(c0, col0, n_valid);
+        process(c1, col0 + 32, n_valid - 32);
+        process(c2, col0 + 64, n_valid - 64);
+        if (half == 0) process(c3, col0 + 96, n_valid - 96);
         if (trace && lane == 0 && n_ev < 128) { trace[3 * n_ev] = tr0; trace[3 * n_ev + 1] = tr1; trace[3 * n_ev + 2] = clock64(); ++n_ev; }
       }
 
@@ -650,12 +698,8 @@ name_topk_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
       long long* o = p.prof + (size_t)pair * 32;
       o[8] = clock64() - pf_t0; o[9] = pf_w; o[10] = pf_fin;
     }
+    teardown();
   }
-
-  // teardown: nobody may free TMEM / exit while the peer can still touch this CTA's memory
-  ptx::tc_fence_before_sync();
-  ptx::cluster_sync_all();
-  if (warp == 2) ptx::tmem_dealloc<2>(tmem_base, kTmemCols);
 }
 
 // Merge `parts` partial top-k lists per row (vocabulary chunks of one GPU: IdxT=int, raw accumulators;

@@ -168,6 +168,22 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity, int tag
   }
 }
 
+// Same bounded wait without a function call on the timeout path: a kernel that moves registers between warp roles
+// with setmaxnreg must not call functions (printf is one), or ptxas compiles every role at the launch register count.
+// The timed-out wait's tag is left in g_mbar_timeout_tag (best effort: the trap may end the grid before it lands).
+__device__ int g_mbar_timeout_tag;
+__device__ __forceinline__ void mbar_wait_nocall(uint32_t bar, uint32_t parity, int tag = 0) {
+  if (mbar_try_wait(bar, parity)) return;
+  WaitClock clk;
+  while (!mbar_try_wait(bar, parity)) {
+    if (clk.expired()) {
+      *reinterpret_cast<volatile int*>(&g_mbar_timeout_tag) = tag;
+      __threadfence();
+      __trap();
+    }
+  }
+}
+
 __device__ __forceinline__ void mbar_wait2(uint32_t bar0, uint32_t bar1, uint32_t parity, int tag = 0) {
   if (mbar_try_wait2(bar0, bar1, parity)) return;
   WaitClock clk;
@@ -375,6 +391,32 @@ __device__ __forceinline__ void tmem_ld_wait(uint32_t (&r)[32]) {
                  "+r"(r[24]), "+r"(r[25]), "+r"(r[26]), "+r"(r[27]), "+r"(r[28]), "+r"(r[29]), "+r"(r[30]), "+r"(r[31])
                :
                : "memory");
+}
+
+// The 32 registers of a tcgen05.ld that an earlier tcgen05.wait::ld has already covered pass through an empty statement:
+// every use of them stays below that wait (one real wait for several loads in flight).
+__device__ __forceinline__ void tmem_ld_keep(uint32_t (&r)[32]) {
+  asm volatile(""
+               : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]),
+                 "+r"(r[8]), "+r"(r[9]), "+r"(r[10]), "+r"(r[11]), "+r"(r[12]), "+r"(r[13]), "+r"(r[14]), "+r"(r[15]),
+                 "+r"(r[16]), "+r"(r[17]), "+r"(r[18]), "+r"(r[19]), "+r"(r[20]), "+r"(r[21]), "+r"(r[22]), "+r"(r[23]),
+                 "+r"(r[24]), "+r"(r[25]), "+r"(r[26]), "+r"(r[27]), "+r"(r[28]), "+r"(r[29]), "+r"(r[30]), "+r"(r[31])
+               :
+               : "memory");
+}
+
+// ------------------------------------------------------------------ register reallocation
+// Per-thread register budget of the executing warpgroup (all four warps execute the same instruction): .dec hands
+// registers back to the CTA's pool, .inc waits until the pool can give them.  N is a multiple of 8 in [24, 256].
+template <int N>
+__device__ __forceinline__ void setmaxnreg_inc() {
+  static_assert(N % 8 == 0 && N >= 24 && N <= 256, "setmaxnreg count");
+  asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(N));
+}
+template <int N>
+__device__ __forceinline__ void setmaxnreg_dec() {
+  static_assert(N % 8 == 0 && N >= 24 && N <= 256, "setmaxnreg count");
+  asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(N));
 }
 
 // ------------------------------------------------------------------ descriptors

@@ -656,7 +656,8 @@ int scd_name_topk(const scd_bf16_t* X, int64_t N, int D, const scd_bf16_t* Wt, i
 
   CUtensorMap mx, mw;
   if (int e = make_map_2d(&mx, X, (uint64_t)N, (uint64_t)D, scd::kBlockM, scd::kAKBlock, CU_TENSOR_MAP_SWIZZLE_128B)) return e;
-  if (int e = make_map_2d(&mw, Wt, (uint64_t)V, (uint64_t)D, scd::kTileN / 2, scd::kAKBlock, CU_TENSOR_MAP_SWIZZLE_128B)) return e;
+  // vocabulary stages are 32-k halves of a k-block: 64-byte rows
+  if (int e = make_map_2d(&mw, Wt, (uint64_t)V, (uint64_t)D, scd::kTileN / 2, scd::kBStageK, CU_TENSOR_MAP_SWIZZLE_64B)) return e;
 
   uint8_t* w8 = reinterpret_cast<uint8_t*>(ws);
   scd::NameParams p;

@@ -154,15 +154,17 @@ def step_name_prof():
     full = prof.cpu()
     p = full[:74 * 32].view(74, 32).double()
     names = {0: 'issuer total', 1: 'issuer wait tmem_empty', 2: 'issuer wait a_full', 3: 'issuer wait b_full (blocking)',
-             4: 'issuer wait token', 5: 'tiles', 6: 'B producer 0 total', 7: 'B producer 0 wait empty', 12: 'B producer 1 total', 13: 'B producer 1 wait empty', 23: 'peer B producer 0 wait empty', 29: 'peer B producer 1 wait empty',
-             14: 'issuer b waits > 150 cyc (count)', 15: 'issuer b waits > 150 cyc (cycles)', 16: 'issuer longest b wait',
+             4: 'issuer wait token', 5: 'tiles', 6: 'B producer 0 total', 7: 'B producer 0 wait empty', 12: 'B producer 1 total',
+             13: 'B producer 1 wait empty', 14: 'B producer 2 total', 15: 'B producer 2 wait empty',
+             23: 'peer B producer 0 wait empty', 29: 'peer B producer 1 wait empty', 31: 'peer B producer 2 wait empty',
              8: 'epi total', 9: 'epi wait tmem_full', 10: 'epi item-final scan'}
     for k, nm in names.items():
         col = p[:, k]
         print(f'{nm:32s} mean={col.mean():12.0f} min={col.min():12.0f} max={col.max():12.0f}')
+    _print_issuer_shares_and_clock(p)
     print('issuer busy-issue cycles per tile:', float(((p[:, 0] - p[:, 1] - p[:, 2] - p[:, 3] - p[:, 4]) / p[:, 5]).mean()))
     print('per-pair issuer total (first 10):', p[:10, 0].tolist())
-    tr = full[74 * 32:].view(4, 128, 3)
+    tr = full[74 * 32:74 * 32 + 4 * 384].view(4, 128, 3)      # the last 384 entries are the per-item timeline
     t0 = int(tr[0, 0, 0])
     print('trace pair 0 (cycles since first event): issuer0 / issuer1 runs: ready, token, issued')
     for i in range(30, 48):
@@ -173,6 +175,35 @@ def step_name_prof():
         a = tr[2, i].tolist()
         print(f'  tile {i}: full {a[0]-t0:8d} released {a[1]-t0:8d} (+{a[1]-a[0]}) done {a[2]-t0:8d} (+{a[2]-a[0]})')
     print('producer 0 issue times:', [int(tr[3, i, 0]) - t0 for i in range(24, 44)])
+
+
+def _gpu_query():
+    """Card name, power limit and maximum SM clock (a query only; it changes no setting)."""
+    import subprocess
+    try:
+        out = subprocess.run(['nvidia-smi', '--query-gpu=name,power.limit,clocks.max.sm', '--format=csv,noheader'],
+                             capture_output=True, text=True, timeout=30).stdout.strip()
+    except (OSError, subprocess.SubprocessError) as e:
+        out = f'(nvidia-smi unavailable: {e})'
+    print('gpu:', out)
+
+
+def _print_issuer_shares_and_clock(p, launch_ms=None):
+    """Issuer waits as shares of the issuer's cycles, and the effective SM clock of the launch: the issuer's clock64
+    span over its %globaltimer span (column 17, ns).  A build that does not record the span gets the cycles over the
+    timed launch (`launch_ms`, which includes the merge and launch gaps: a lower bound on the clock)."""
+    tot = p[:, 0].sum()
+    te, bf, tok = p[:, 1].sum() / tot, p[:, 3].sum() / tot, p[:, 4].sum() / tot
+    print(f'issuer shares: tmem_empty {100 * te:.1f} %  b_full {100 * bf:.1f} %  tmem_empty + b_full {100 * (te + bf):.1f} %  '
+          f'token {100 * tok:.1f} %')
+    ns = p[:, 17]
+    if float(ns.min()) > 0:
+        mhz = p[:, 0] / ns * 1e3
+        print(f'effective SM clock: mean {float(mhz.mean()):.0f} MHz  min {float(mhz.min()):.0f}  max {float(mhz.max()):.0f} '
+              f'(issuer span {float(ns.mean()) / 1e3:.1f} us)')
+    elif launch_ms:
+        print(f'effective SM clock >= {float(p[:, 0].mean()) / (launch_ms * 1e3):.0f} MHz (issuer cycles / timed launch; span not recorded)')
+    _gpu_query()
 
 
 def step_estep_prof():
@@ -308,6 +339,7 @@ def step_name_items():
                       5: 'tiles', 8: 'epi total', 9: 'epi wait tmem_full', 10: 'epi item-final scan+write'}.items():
             col = p[:, k]
             print(f'   {nm:28s} mean={col.mean():11.0f} min={col.min():11.0f} max={col.max():11.0f}')
+        _print_issuer_shares_and_clock(p[p[:, 0] > 0], ms)
         it = full[74 * 32 + 4 * 384:].view(64, 6)
         t0 = int(it[0, 0]) if int(it[0, 0]) else int(it[0, 1])
         print('   pair 0 items: first MMA | first tile seen | tiles done | scan done | results written | A loads issued   (cycles since the first MMA)')
