@@ -55,8 +55,7 @@ SCD_API int scd_pairwise_distance(const float* X, int64_t N, int D, const float*
  * ws holds the per-iteration centroid hi/lo planes and norms; they are recomputed from C by a small kernel unless
  * SCD_ESTEP_PLANES_READY says the previous scd_finalize_centers already left them there. */
 #define SCD_ESTEP_EXACT 1          /* force the fp32 direct-form kernel */
-#define SCD_ESTEP_PLANES_READY 2
-#define SCD_ESTEP_ACCUMULATE 4     /* scd_estep_mstep: add to sums / counts as they are (row panels of one iteration) */   /* ws already holds the operands of C: scd_finalize_centers(estep_ws = ws) wrote them */
+#define SCD_ESTEP_PLANES_READY 2   /* ws already holds the operands of C: scd_finalize_centers(estep_ws = ws) wrote them */
 SCD_API size_t scd_estep_workspace_bytes(int K, int D);
 /* 1 when (N, D, K) takes the tensor-core path (given an aligned X and a workspace) - what the host layer needs to know
  * before it asks scd_finalize_centers to prepare the next E-step's operands. */
@@ -64,15 +63,6 @@ SCD_API int scd_estep_uses_tensor_cores(int64_t N, int D, int K);
 SCD_API int scd_estep(const float* X, int64_t N, int D, const float* C, int K,
               int64_t* labels, float* mindist /* nullable */, double* inertia_acc /* nullable */, int flags,
               void* ws, size_t ws_bytes, scd_stream_t stream);
-/* faster_mix_k_means_pytorch.py:58-64 in ONE pass over X: scd_estep that also accumulates the M-step's per-cluster sums
- * ([K,D] fp32) and counts ([K] int32; both zeroed here first unless SCD_ESTEP_ACCUMULATE) - the rows of a tile are re-read from L2 right after their
- * argmin and added to sums[label] with vector reductions, so X leaves HBM once per iteration and no label sort is needed.
- * Only where scd_estep_fused_supported(N, D, K) (tensor-core E-step plan with room for the staging rows: K <= 256).
- * Follow with scd_finalize_centers (or its _peer variant: sums / counts may live in a peer-mapped exchange block). */
-SCD_API int scd_estep_fused_supported(int64_t N, int D, int K);
-SCD_API int scd_estep_mstep(const float* X, int64_t N, int D, const float* C, int K, int64_t* labels, float* mindist /* nullable */,
-                    double* inertia_acc /* nullable */, int flags, float* sums, int32_t* counts, void* ws, size_t ws_bytes,
-                    scd_stream_t stream);
 
 /* k-means++ seeding, faster_mix_k_means_pytorch.py:20-36 (gcd copy :82-110), without the per-centre N x c distance
  * matrix and without a host round trip per centre:

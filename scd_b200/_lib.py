@@ -22,8 +22,6 @@ SIGNATURES = {
     'scd_estep_workspace_bytes': (_sz, [_int, _int]),
     'scd_estep_uses_tensor_cores': (_int, [_i64, _int, _int]),
     'scd_estep': (_int, [_vp, _i64, _int, _vp, _int, _vp, _vp, _vp, _int, _vp, _sz, _vp]),
-    'scd_estep_fused_supported': (_int, [_i64, _int, _int]),
-    'scd_estep_mstep': (_int, [_vp, _i64, _int, _vp, _int, _vp, _vp, _vp, _int, _vp, _vp, _vp, _sz, _vp]),
     'scd_kpp_workspace_bytes': (_sz, [_i64]),
     'scd_kpp_update': (_int, [_vp, _i64, _int, _vp, _vp, _int, _vp, _vp, _vp, _sz, _vp]),
     'scd_kpp_select': (_int, [_vp, _i64, _int, C.c_double, _vp, _vp, _vp, _sz, _vp]),
@@ -59,7 +57,7 @@ SIGNATURES = {
     'scd_linear_assignment': (_int, [_vp, _int, _int, _vp, C.POINTER(_int)]),
 }
 
-ESTEP_EXACT, ESTEP_PLANES_READY, ESTEP_ACCUMULATE = 1, 2, 4          # scd_estep flags (include/scd_b200.h)
+ESTEP_EXACT, ESTEP_PLANES_READY = 1, 2          # scd_estep flags (include/scd_b200.h)
 
 _lib = None
 

@@ -50,12 +50,8 @@ constexpr int kEsConvSets = 2;          // converter warp sets (4 warps each), a
 constexpr int kEsIssuers = 3;           // MMA issuer warps (1, 16, 17), k-blocks round-robin
 constexpr int kEsFirstExtraIssuer = 4 + 4 * kEsConvSets + 4;       // warps 16, 17
 constexpr int kEsSecondCProducer = kEsFirstExtraIssuer + kEsIssuers - 1;   // warp 18
-constexpr int kEsMWarp = kEsSecondCProducer + 1;                   // warp 19: fused M-step (segment sums of the tile just assigned)
-constexpr int kEsThreads = 32 * (kEsMWarp + 1);                    // 640: five warps per scheduler, still 96 registers
+constexpr int kEsThreads = 32 * (kEsSecondCProducer + 1);          // 608: one scheduler holds five warps, so still 96 registers
 constexpr int kEsMaxK = 1024;
-constexpr int kEsMaxMStages = 16;       // staging rows of the fused M-step in flight (host picks EsParams::m_stages)
-// fused M-step region of shared memory: [cluster counts: kEsMaxK ints][labels of two tiles: 2 x 128 ints][staging rows]
-constexpr int kEsMCntOff = 0, kEsMLabOff = 4 * kEsMaxK, kEsMHeader = 4 * kEsMaxK + 2 * 4 * kEsBM;
 
 // Dynamic shared memory: [X ring: x_stages x 16 KB][A ring: 3 x (hi, lo) x 8 KB, kTmemA = false only][B ring: 3 x (hi, lo) x b_plane]
 // [tail: barriers, TMEM pointer, ||c||^2, ||x||^2 ring].  The E-step is HBM-latency bound (ncu, round 1: the
@@ -73,11 +69,7 @@ struct EsTail {
   static constexpr int tmem_ptr = drain + 16;
   static constexpr int cnorm = tmem_ptr + 16;                                   // [kEsMaxK] floats
   static constexpr int xnorm = cnorm + 4 * kEsMaxK;                             // [4 tiles][sets][128] floats
-  // fused M-step (EsParams::sums != nullptr): labels of the two tiles in flight, per-CTA cluster counts, barriers
-  static constexpr int lab_full = xnorm + 4 * 4 * kEsConvSets * kEsBM;          // [2]
-  static constexpr int lab_empty = lab_full + 16;                               // [2]
-  static constexpr int m_full = lab_empty + 16;                                 // [16] staging rows
-  static constexpr int total = m_full + 8 * kEsMaxMStages;
+  static constexpr int total = xnorm + 4 * 4 * kEsConvSets * kEsBM;
 };
 constexpr int kEsSmemLimit = 232448;    // 227 KB opt-in maximum per CTA
 
@@ -98,25 +90,16 @@ struct EsParams {
   float* mindist;          // nullable [N]
   double* inertia;         // nullable
   long long* prof;         // nullable: [CTAs][16] cycle counters (scd_debug_set_name_profile), debugging aid
-  // fused M-step (faster_mix_k_means_pytorch.py:61-64 in the same pass): nullable.  sums [K, D] fp32 and counts [K] int32
-  // are ACCUMULATED into (the caller zeroes them): row i is added to sums[labels[i]] right after its tile's argmin
-  float* sums;
-  int* counts;
-  const float* x;          // [N, d] fp32, the rows map_x describes
-  int d;
-  int m_stages;            // staging rows in flight (0: no fused M-step)
-  int m_row_bytes;         // d * 4 rounded up to 128
 };
 
 // host + device: byte offsets of the rings for a given plan
 struct EsLayout {
-  int x_off, a_off, b_off, m_off, tail_off, total;
-  __host__ __device__ EsLayout(int x_stages, int b_plane, bool tmem_a, int m_stages = 0, int m_row_bytes = 0) {
+  int x_off, a_off, b_off, tail_off, total;
+  __host__ __device__ EsLayout(int x_stages, int b_plane, bool tmem_a) {
     x_off = 0;
     a_off = x_off + x_stages * kEsXBytes;
     b_off = a_off + (tmem_a ? 0 : kEsAStages * 2 * kEsAPlane);
-    m_off = b_off + es_b_stages(tmem_a) * 2 * b_plane;
-    tail_off = m_off + (m_stages > 0 ? kEsMHeader + m_stages * m_row_bytes : 0);
+    tail_off = b_off + es_b_stages(tmem_a) * 2 * b_plane;
     total = tail_off + EsTail::total;
   }
 };
@@ -169,8 +152,7 @@ estep_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant
   const uint32_t warp = threadIdx.x >> 5;
   const uint32_t lane = threadIdx.x & 31;
   const int nkb = p.num_kb;
-  const EsLayout L(p.x_stages, p.b_plane, kTmemA, p.m_stages, p.m_row_bytes);
-  const bool fused_m = p.sums != nullptr;
+  const EsLayout L(p.x_stages, p.b_plane, kTmemA);
   const int kEsXStages = p.x_stages;
   const int n_as = p.a_stages;
   constexpr uint32_t kNB = (uint32_t)es_b_stages(kTmemA);      // centroid ring depth
@@ -195,8 +177,6 @@ estep_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant
     for (int s = 0; s < kNB; ++s) { ptx::mbar_init(bar(EsTail::b_full, s), 1); ptx::mbar_init(bar(EsTail::b_empty, s), 1); }
     for (int b = 0; b < 2; ++b) { ptx::mbar_init(bar(EsTail::t_full, b), 1); ptx::mbar_init(bar(EsTail::t_empty, b), 4); }
     ptx::mbar_init(bar(EsTail::drain, 0), kEsIssuers);
-    for (int b = 0; b < 2; ++b) { ptx::mbar_init(bar(EsTail::lab_full, b), 4); ptx::mbar_init(bar(EsTail::lab_empty, b), 1); }
-    for (int s2 = 0; s2 < kEsMaxMStages; ++s2) ptx::mbar_init(bar(EsTail::m_full, s2), 1);
     ptx::fence_mbar_init_cluster();
   }
   if (warp == 2) {
@@ -206,8 +186,6 @@ estep_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant
   {
     float* cn = reinterpret_cast<float*>(smem + L.tail_off + EsTail::cnorm);
     for (int k = threadIdx.x; k < p.n_clusters; k += blockDim.x) cn[k] = p.cnorm[k];
-    int* cnt = reinterpret_cast<int*>(smem + L.m_off + kEsMCntOff);
-    if (fused_m) for (int k = threadIdx.x; k < p.n_clusters; k += blockDim.x) cnt[k] = 0;
   }
   ptx::tc_fence_before_sync();
   __syncthreads();
@@ -232,7 +210,7 @@ estep_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant
             twait(bar(EsTail::x_empty, xs), xph ^ 1, 700 + xs, w_xe);
             ptx::mbar_arrive_expect_tx(bar(EsTail::x_full, xs), kEsXBytes);
             ptx::tma_load_2d<1>(sbase + L.x_off + xs * kEsXBytes, &map_x, bar(EsTail::x_full, xs), kb * kEsBK, rt * kEsBM,
-                                (p.n_ntiles > 1 || fused_m) ? ptx::kEvictNormal : ptx::kEvictFirst);   // fused: re-read from L2 soon
+                                p.n_ntiles > 1 ? ptx::kEvictNormal : ptx::kEvictFirst);
           }
         }
       }
@@ -548,16 +526,6 @@ estep_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant
         if (p.mindist) p.mindist[row] = d;
         inertia_local += (double)d;
       }
-      if (fused_m) {
-        // hand the tile's labels to the M-step warp (slot = tile parity; it released the slot two tiles ago)
-        const uint32_t ls = my_tile & 1u;
-        if (my_tile >= 2) ptx::mbar_wait(bar(EsTail::lab_empty, ls), ((my_tile >> 1) & 1u) ^ 1u, 780 + ls);
-        const bool ok = row < p.n_rows && best_k >= 0 && best_k < p.n_clusters;
-        reinterpret_cast<int*>(smem + L.m_off + kEsMLabOff)[ls * kEsBM + row_in_tile] = ok ? best_k : -1;
-        if (ok) atomicAdd(reinterpret_cast<int*>(smem + L.m_off + kEsMCntOff) + best_k, 1);
-        __syncwarp();
-        if (lane == 0) ptx::mbar_arrive(bar(EsTail::lab_full, ls));
-      }
     }
     if (prof && warp == 4 + 4 * kEsConvSets && lane == 0) pf[10] = w_tf;
     if (p.inertia) {
@@ -566,67 +534,9 @@ estep_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant
     }
   }
 
-  else if (warp == kEsMWarp && fused_m) {
-    // =================================================== fused M-step: sums[label] += row, for the tile just assigned
-    // The tile's rows were streamed through L2 a few microseconds ago: they come back with asynchronous 16-byte copies
-    // (cp.async: no registers held, m_stages rows in flight; one warp issuing TMA bulk copies instead gets one copy per
-    // ~1300 cycles, 8 x too slow - measured) into a ring of staging rows, and the warp adds each row to its cluster's sum
-    // with red.global.add.v4.f32 (512 bytes per instruction, fire and forget).  Lane l copies and reduces the same 16
-    // bytes of every 512-byte slice, so no cross-lane visibility is involved.  No sort, no second pass over X in HBM:
-    // 24.4 M vector reductions per C2 pass, which the L2 absorbs in ~100 us while the E-step streams
-    // (tools/red_scatter_bench.cu) - about the E-step's own duration.
-    const int S = p.m_stages;
-    const int* lab_s = reinterpret_cast<const int*>(smem + L.m_off + kEsMLabOff);
-    const uint32_t stage0 = sbase + L.m_off + kEsMHeader;
-    const uint8_t* const stage0_p = smem + L.m_off + kEsMHeader;
-    const int nvec = (p.d + 127) >> 7;
-    uint32_t q_load = 0, q_use = 0;           // rows whose copies have been issued / that have been consumed, over the whole kernel
-    uint32_t my_tile = 0;
-    for (int rt = blockIdx.x; rt < p.n_row_tiles; rt += gridDim.x, ++my_tile) {
-      const uint32_t ls = my_tile & 1u;
-      ptx::mbar_wait(bar(EsTail::lab_full, ls), (my_tile >> 1) & 1u, 800 + ls);
-      const long long row0 = (long long)rt * kEsBM;
-      const int n_here = (int)min((long long)kEsBM, p.n_rows - row0);
-      auto issue_row = [&](int r) {            // all lanes: row r of this tile -> staging slot q_load % S, one group
-        const uint32_t dst = stage0 + (q_load % (uint32_t)S) * (uint32_t)p.m_row_bytes;
-        const float* src = p.x + (size_t)(row0 + r) * p.d;
-        for (int j = 0; j < nvec; ++j) {
-          const int c = j * 128 + (int)lane * 4;
-          if (c < p.d) ptx::cp_async_16(dst + (uint32_t)c * 4u, src + c);
-        }
-        ptx::cp_async_commit();
-        ++q_load;
-      };
-      int issued = 0;
-      for (; issued < min(S, n_here); ++issued) issue_row(issued);
-      for (int r = 0; r < n_here; ++r, ++q_use) {
-        ptx::cp_async_wait_dyn(issued - r - 1);            // groups issued after row r's may still be in flight
-        const int lab = lab_s[ls * kEsBM + r];
-        const float* src = reinterpret_cast<const float*>(stage0_p + (q_use % (uint32_t)S) * (uint32_t)p.m_row_bytes);
-        if (lab >= 0) {
-          float* dst = p.sums + (size_t)lab * p.d;
-          for (int j = 0; j < nvec; ++j) {
-            const int c = j * 128 + (int)lane * 4;
-            if (c < p.d) {
-              const float4 v = *reinterpret_cast<const float4*>(src + c);
-              asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst + c), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
-            }
-          }
-        }
-        if (issued < n_here) { issue_row(issued); ++issued; }       // the slot just read is free again (same lane, program order)
-      }
-      __syncwarp();
-      if (lane == 0) ptx::mbar_arrive(bar(EsTail::lab_empty, ls));
-    }
-  }
-
   ptx::tc_fence_before_sync();
   __syncthreads();
   if (warp == 2) ptx::tmem_dealloc<1>(tmem_base, 512);
-  if (fused_m && p.counts) {                    // this CTA's cluster counts
-    const int* cnt = reinterpret_cast<const int*>(smem + L.m_off + kEsMCntOff);
-    for (int k = threadIdx.x; k < p.n_clusters; k += blockDim.x) { const int c = cnt[k]; if (c) atomicAdd(p.counts + k, c); }
-  }
 }
 
 }  // namespace scd

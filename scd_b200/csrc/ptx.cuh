@@ -228,32 +228,6 @@ __device__ __forceinline__ void bulk_load_1d(uint32_t smem_dst, const void* gsrc
       ::"r"(smem_dst), "l"(gsrc), "r"(bytes), "r"(bar), "l"(hint)
       : "memory");
 }
-// Ampere-style asynchronous copy global -> shared, 16 bytes per thread, L1 bypassed; groups complete in order
-__device__ __forceinline__ void cp_async_16(uint32_t smem_dst, const void* gsrc) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_dst), "l"(gsrc) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-// wait until at most n (0..15) of this thread's most recent groups are still in flight
-__device__ __forceinline__ void cp_async_wait_dyn(int n) {
-  switch (n) {
-    case 0: asm volatile("cp.async.wait_group 0;" ::: "memory"); break;
-    case 1: asm volatile("cp.async.wait_group 1;" ::: "memory"); break;
-    case 2: asm volatile("cp.async.wait_group 2;" ::: "memory"); break;
-    case 3: asm volatile("cp.async.wait_group 3;" ::: "memory"); break;
-    case 4: asm volatile("cp.async.wait_group 4;" ::: "memory"); break;
-    case 5: asm volatile("cp.async.wait_group 5;" ::: "memory"); break;
-    case 6: asm volatile("cp.async.wait_group 6;" ::: "memory"); break;
-    case 7: asm volatile("cp.async.wait_group 7;" ::: "memory"); break;
-    case 8: asm volatile("cp.async.wait_group 8;" ::: "memory"); break;
-    case 9: asm volatile("cp.async.wait_group 9;" ::: "memory"); break;
-    case 10: asm volatile("cp.async.wait_group 10;" ::: "memory"); break;
-    case 11: asm volatile("cp.async.wait_group 11;" ::: "memory"); break;
-    case 12: asm volatile("cp.async.wait_group 12;" ::: "memory"); break;
-    case 13: asm volatile("cp.async.wait_group 13;" ::: "memory"); break;
-    case 14: asm volatile("cp.async.wait_group 14;" ::: "memory"); break;
-    default: asm volatile("cp.async.wait_group 15;" ::: "memory"); break;
-  }
-}
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
 __device__ __forceinline__ void tma_load_3d(uint32_t smem_dst, const void* desc, uint32_t bar, int c0, int c1, int c2, uint64_t hint) {

@@ -290,46 +290,9 @@ size_t scd_estep_workspace_bytes(int K, int D) {
   return align_up((size_t)K * D * 2, 256) * 2 + align_up((size_t)K * sizeof(float), 256) + 256;
 }
 
-// smallest X ring the fused plan keeps, and the staging depth it wants per centroid-tile count (a tile of K > 256 clusters
-// takes n_ntiles accumulator passes, so its M-step has that much longer)
-constexpr int kFusedMinXStages = 4;
-
-static int plan_fused_stages(int D, int K, int* x_stages_out) {
-  const int n_ntiles = (K + 255) / 256;
-  const int n_tile = n_ntiles > 1 ? 256 : ((K + 15) / 16) * 16;
-  const int num_kb = (D + scd::kEsBK - 1) / scd::kEsBK;
-  const bool tmem_a = n_ntiles == 1 && n_tile + 3 * 32 <= 256 && num_kb >= 3;
-  const int b_plane = n_tile * scd::kEsBK * 2;
-  const int row_bytes = ((D * 4 + 127) / 128) * 128;
-  const int fixed = scd::EsLayout(0, b_plane, tmem_a).total + 1024 + scd::kEsMHeader;
-  // as many staging rows as fit next to an X ring of at least kFusedMinXStages (preferably 6) stages
-  for (int want_x : {6, kFusedMinXStages}) {
-    const int left = scd::kEsSmemLimit - fixed - want_x * scd::kEsXBytes;
-    int m = std::min(scd::kEsMaxMStages, left / row_bytes);
-    const int need = n_ntiles > 1 ? 4 : 8;
-    if (m >= need) {
-      m = std::min(m, n_ntiles > 1 ? 8 : scd::kEsMaxMStages);
-      if (x_stages_out) {
-        int xs = (scd::kEsSmemLimit - fixed - m * row_bytes) / scd::kEsXBytes;
-        *x_stages_out = std::max(2, std::min(scd::kEsMaxXStages, xs)) & ~1;
-      }
-      return m;
-    }
-  }
-  return 0;
-}
-
-int scd_estep_fused_supported(int64_t N, int D, int K) {
-  return scd_estep_uses_tensor_cores(N, D, K) && D % 4 == 0 && plan_fused_stages(D, K, nullptr) > 0 ? 1 : 0;
-}
-
-static int estep_impl(const float* X, int64_t N, int D, const float* C, int K, int64_t* labels, float* mindist, double* inertia_acc,
-                      int flags, float* sums, int32_t* counts, void* ws, size_t ws_bytes, scd_stream_t stream) {
+int scd_estep(const float* X, int64_t N, int D, const float* C, int K, int64_t* labels, float* mindist, double* inertia_acc,
+              int flags, void* ws, size_t ws_bytes, scd_stream_t stream) {
   if (N < 0 || D <= 0 || K <= 0) return fail("scd_estep: bad shape N=%lld D=%d K=%d", (long long)N, D, K);
-  if (sums && counts && !(flags & SCD_ESTEP_ACCUMULATE)) {                 // fused M-step accumulates: start from zero
-    SCD_CUDA(cudaMemsetAsync(sums, 0, sizeof(float) * (size_t)K * D, as_stream(stream)));
-    SCD_CUDA(cudaMemsetAsync(counts, 0, sizeof(int32_t) * (size_t)K, as_stream(stream)));
-  }
   if (N == 0) return 0;
   if (!X || !C || !labels) return fail("scd_estep: null pointer");
   const bool exact = (flags & SCD_ESTEP_EXACT) != 0;
@@ -338,8 +301,6 @@ static int estep_impl(const float* X, int64_t N, int D, const float* C, int K, i
   // warp set must own at least one k-block per tile (it publishes its share of ||x||^2 there)
   const bool tc_ok = !exact && scd_estep_uses_tensor_cores(N, D, K) && (reinterpret_cast<uintptr_t>(X) & 15) == 0 && ws &&
                      ws_bytes >= scd_estep_workspace_bytes(K, D);
-  if (sums && !(tc_ok && scd_estep_fused_supported(N, D, K)))
-    return fail("scd_estep_mstep: the fused M-step needs the tensor-core E-step plan (see scd_estep_fused_supported)");
   if (!tc_ok) {
     dim3 grid((unsigned)((N + scd::kDistBM - 1) / scd::kDistBM));
     scd::sqdist_kernel<true><<<grid, scd::kDistThreads, 0, st>>>(X, N, D, C, K, nullptr, nullptr,
@@ -369,12 +330,6 @@ static int estep_impl(const float* X, int64_t N, int D, const float* C, int K, i
   p.mindist = mindist;
   p.inertia = inertia_acc;
   p.prof = g_name_prof;
-  p.sums = sums;
-  p.counts = counts;
-  p.x = X;
-  p.d = D;
-  p.m_stages = 0;
-  p.m_row_bytes = ((D * 4 + 127) / 128) * 128;
   CUtensorMap mx, mc;
   if (int e = make_map_2d(&mx, X, (uint64_t)N, (uint64_t)D, scd::kEsBM, scd::kEsBK, CU_TENSOR_MAP_SWIZZLE_128B, true)) return e;
   // hi and lo planes as one 3-D tensor [2][K][D]: a single box brings both k-slabs of a stage
@@ -396,12 +351,7 @@ static int estep_impl(const float* X, int64_t N, int D, const float* C, int K, i
     // for K = 200 / 208 / 224 (five stages) until this was found with tools/estep_stress2.py.
     p.x_stages &= ~1;
   }
-  if (sums) {                               // fused M-step: staging rows take the place of some X stages
-    int xs = 0;
-    p.m_stages = plan_fused_stages(D, K, &xs);
-    p.x_stages = xs;
-  }
-  const int smem = scd::EsLayout(p.x_stages, p.b_plane, tmem_a, p.m_stages, p.m_row_bytes).total + 1024;
+  const int smem = scd::EsLayout(p.x_stages, p.b_plane, tmem_a).total + 1024;
   if (smem > scd::kEsSmemLimit) return fail("scd_estep: shared-memory plan does not fit (%d bytes)", smem);
   static int attr_smem[kMaxDevices][2] = {};
   const int dev = current_device_slot();
@@ -415,18 +365,6 @@ static int estep_impl(const float* X, int64_t N, int D, const float* C, int K, i
   else scd::estep_tc_kernel<false><<<grid, scd::kEsThreads, smem, st>>>(mx, mc, p);
   SCD_LAUNCH_CHECK("estep_tc_kernel");
   return 0;
-}
-
-int scd_estep(const float* X, int64_t N, int D, const float* C, int K, int64_t* labels, float* mindist, double* inertia_acc,
-              int flags, void* ws, size_t ws_bytes, scd_stream_t stream) {
-  return estep_impl(X, N, D, C, K, labels, mindist, inertia_acc, flags, nullptr, nullptr, ws, ws_bytes, stream);
-}
-
-int scd_estep_mstep(const float* X, int64_t N, int D, const float* C, int K, int64_t* labels, float* mindist, double* inertia_acc,
-                    int flags, float* sums, int32_t* counts, void* ws, size_t ws_bytes, scd_stream_t stream) {
-  if (!sums || !counts) return fail("scd_estep_mstep: null sums / counts");
-  if (flags & SCD_ESTEP_EXACT) return fail("scd_estep_mstep: the exact fp32 E-step has no fused M-step");
-  return estep_impl(X, N, D, C, K, labels, mindist, inertia_acc, flags, sums, counts, ws, ws_bytes, stream);
 }
 
 // ---------------------------------------------------------------------------- k-means++ seeding (a5)

@@ -53,21 +53,16 @@ class _EStep:
         self.ready_for = None
 
     def fusable(self, n):
-        """True when ``run(..., mstep=...)`` can accumulate the M-step's sums in the same pass (``scd_estep_mstep``)."""
-        return bool(_lib.load().scd_estep_fused_supported(max(int(n), 1), self.d, self.k))
+        """Always False: the one-pass E+M kernel was removed (DESIGN 3.3).  Kept for ``bench.py --fused-em``, its only
+        caller, which then runs the two-pass round."""
+        return False
 
-    def run(self, X, C, labels_out, inertia_acc, mindist=None, exact=False, mstep: '_MStep | None' = None, accumulate=False):
+    def run(self, X, C, labels_out, inertia_acc, mindist=None, exact=False):
         lib = _lib.load()
-        flags = (_lib.ESTEP_EXACT if exact else 0) | (_lib.ESTEP_ACCUMULATE if accumulate else 0)
+        flags = _lib.ESTEP_EXACT if exact else 0
         if self.ready_for is not None and self.ready_for == C.data_ptr():
             flags |= _lib.ESTEP_PLANES_READY
         self.ready_for = None
-        if mstep is not None:               # E-step + M-step sums in one pass over X (the caller has checked fusable())
-            _lib.check(lib.scd_estep_mstep(X.data_ptr(), X.shape[0], X.shape[1], C.data_ptr(), C.shape[0], labels_out.data_ptr(),
-                                           _lib.ptr(mindist), _lib.ptr(inertia_acc), flags, mstep.sums.data_ptr(),
-                                           mstep.counts.data_ptr(), self.ws.data_ptr(), self.ws.numel(), _stream()), 'scd_estep_mstep')
-            mstep.sorted_for = None
-            return
         _lib.check(lib.scd_estep(X.data_ptr(), X.shape[0], X.shape[1], C.data_ptr(), C.shape[0],
                                  labels_out.data_ptr(), _lib.ptr(mindist), _lib.ptr(inertia_acc), flags,
                                  self.ws.data_ptr(), self.ws.numel(), _stream()), 'scd_estep')
@@ -141,14 +136,15 @@ class _MStep:
 PANEL_ROWS = 16384          # rows per upload panel of assign_from_host (50 MB of fp32 at D = 768: ~0.9 ms of PCIe, ~12 us of E-step)
 
 
-def assign_from_host(X_host: torch.Tensor, centers: torch.Tensor, panel_rows: int = PANEL_ROWS, mstep: '_MStep | None' = None):
+def assign_from_host(X_host: torch.Tensor, centers: torch.Tensor, panel_rows: int = PANEL_ROWS, mstep=None):
     """E-step of one iteration (``faster_mix_k_means_pytorch.py:58-60``) on HOST features: ``torch.from_numpy(x).cuda()``
     (``main_unsup.py:340``) and the assignment pipelined - the rows go up in panels on a copy stream and each panel is
     assigned (fused distance + argmin + inertia) while the next one is on the wire, so only the last panel's ~12 us of
     E-step are left after the transfer.  Rows are independent: labels equal the resident launch bit for bit.
-    ``mstep``: an ``_MStep`` for ``(N, D, K)`` - each panel's launch then also accumulates the M-step's sums and counts
-    (``scd_estep_mstep``), so after the last byte only the divide is left (``update_centers(..., mstep=...)``).
+    ``mstep`` must be None: the one-pass E+M that accumulated the M-step's sums per panel was removed (DESIGN 3.3).
     Returns ``(X on the device, labels int64 [N], inertia fp64 [1])``."""
+    if mstep is not None:
+        raise ValueError('assign_from_host: mstep= must be None - the one-pass E+M was removed (DESIGN 3.3)')
     if not torch.is_tensor(X_host):
         X_host = torch.from_numpy(np.ascontiguousarray(X_host))
     if X_host.is_cuda or X_host.dtype != torch.float32 or X_host.dim() != 2:
@@ -173,18 +169,15 @@ def assign_from_host(X_host: torch.Tensor, centers: torch.Tensor, panel_rows: in
         main.wait_event(up)
         if lo:
             es.ready_for = Cd.data_ptr()             # the centroid planes of the first panel's launch are still in place
-        fused = mstep is not None and es.fusable(hi - lo)
-        es.run(X[lo:hi], Cd, labels[lo:hi], inertia, mstep=mstep if fused else None, accumulate=fused and lo > 0)
-        if mstep is not None and not fused:
-            raise ValueError('this (D, K) has no fused E+M plan: call update_centers without mstep=')
+        es.run(X[lo:hi], Cd, labels[lo:hi], inertia)
     X.record_stream(main)
     return X, labels, inertia
 
 
 def update_centers(X: torch.Tensor, labels: torch.Tensor, k: int, c_old: torch.Tensor | None = None, mstep: '_MStep | None' = None):
     """M-step (``faster_mix_k_means_pytorch.py:61-64``): ``centers[j] = mean(X[labels == j])`` on device-resident rows,
-    NaN row for an empty cluster.  ``mstep``: the ``_MStep`` whose sums ``assign_from_host(..., mstep=)`` has already
-    accumulated - only the divide is left.  Returns ``(centers [K, D], counts int32 [K], move norms or None, the _MStep)``."""
+    NaN row for an empty cluster.  ``mstep``: an ``_MStep`` whose ``sums_counts`` has already run on ``(X, labels)`` -
+    only the divide is left.  Returns ``(centers [K, D], counts int32 [K], move norms or None, the _MStep)``."""
     Xd = _dev_f32(X)
     ms = mstep
     if ms is None:
@@ -241,8 +234,6 @@ def predict(X, cluster_centers, batch_size=None):
 class K_Means:
     """Same constructor as the reference (``faster_mix_k_means_pytorch.py:9``; gcd copy appends ``mode``).
     ``process_group`` is the only extension (row-sharded multi-GPU)."""
-
-    _fused_em = True      # the E-step may accumulate the M-step's sums in the same pass (subclasses with another assignment: False)
 
     def __init__(self, k=3, tolerance=1e-4, max_iterations=100, init='k-means++', n_init=10, random_state=None,
                  n_jobs=None, pairwise_batch_size=None, mode=None, *, process_group=None):
@@ -355,13 +346,6 @@ class K_Means:
         best_labels = best_inertia = best_centers = None
         n_done = 0
         u_view = labels[l_num:]
-        # One pass over X per iteration (scd_estep_mstep) is opt-in, SCD_B200_FUSED_EM=1: the L2 absorbs the 24.4 M vector
-        # reductions of a C2 pass in ~86 us at best (profiles/r2_red_scatter_bench.txt, r2_mwarp_bench.txt) - more than the
-        # segment sum's second pass over X costs (68 us) - so two passes stay the default (DESIGN 3.3).
-        import os
-        fuse = (self._fused_em and os.environ.get('SCD_B200_FUSED_EM', '0') == '1' and l_num == 0
-                and X_assign.shape[0] == X_all.shape[0] and X_assign.data_ptr() == X_all.data_ptr()
-                and X_all.shape[0] > 0 and estep.fusable(X_all.shape[0]))
         for it in range(self.max_iterations):
             n_done = it + 1
             if px is not None:                      # this iteration's [sums | counts | inertia] block, mapped by every rank
@@ -369,16 +353,13 @@ class K_Means:
                 mstep.bind_peer(px, block)
                 inertia_acc = block[2]
             inertia_acc.zero_()
-            if fuse:
-                estep.run(X_all, c_cur, labels, inertia_acc, mstep=mstep)          # :58-64 in one pass over X
-            else:
-                if X_assign.shape[0]:
-                    self._assign(X_assign, c_cur, u_view, inertia_acc, estep)      # :58-60 / :105-107,:111
-                if l_num:
-                    lib = _lib.load()
-                    _lib.check(lib.scd_labelled_inertia(l_feats.data_ptr(), labels.data_ptr(), l_num, d, c_cur.data_ptr(), k,
-                                                        inertia_acc.data_ptr(), _stream()), 'scd_labelled_inertia')   # :108-110
-                mstep.sums_counts(X_all, labels)                                   # :61-64 / :113-116
+            if X_assign.shape[0]:
+                self._assign(X_assign, c_cur, u_view, inertia_acc, estep)          # :58-60 / :105-107,:111
+            if l_num:
+                lib = _lib.load()
+                _lib.check(lib.scd_labelled_inertia(l_feats.data_ptr(), labels.data_ptr(), l_num, d, c_cur.data_ptr(), k,
+                                                    inertia_acc.data_ptr(), _stream()), 'scd_labelled_inertia')   # :108-110
+            mstep.sums_counts(X_all, labels)                                       # :61-64 / :113-116
             if px is not None:                      # all-reduce over peer loads + divide + :71 / :123, one launch
                 mstep.finalize_peer(c_cur, c_new, inertia_red, estep=estep if mstep.tc else None)
             else:

@@ -53,8 +53,6 @@ def labels_constrained(cost_x1000, size_min: int, size_max: int):
 class K_Means(_K_Means):
     """Constructor of ``local_utils/sskm_constrained.py:16``."""
 
-    _fused_em = False      # labels come from the size-constrained assignment, not from the E-step's argmin
-
     def __init__(self, k=3, tolerance=1e-4, max_iterations=100, size_min=100, size_max=1000, init='k-means++', n_init=10,
                  random_state=None, n_jobs=None, pairwise_batch_size=None):
         super().__init__(k=k, tolerance=tolerance, max_iterations=max_iterations, init=init, n_init=n_init,

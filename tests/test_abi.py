@@ -44,6 +44,17 @@ def test_workspace_sizes_are_sane_without_a_gpu():
     assert 1000 * 5 * 8 <= small and 127000 * 5 * 8 <= big < 127000 * 5 * 8 * 20
 
 
+def test_removed_one_pass_em_is_refused_without_device_work():
+    """assign_from_host keeps its mstep= keyword but refuses a value before touching the device, and the E-step
+    reports no one-pass E+M plan (called unbound: constructing an _EStep allocates on the device)."""
+    import pytest
+    import torch
+    from scd_b200 import kmeans
+    with pytest.raises(ValueError, match='one-pass E\\+M was removed'):
+        kmeans.assign_from_host(np.zeros((4, 8), np.float32), torch.zeros(2, 8), mstep=object())
+    assert kmeans._EStep.fusable(object(), 127000) is False
+
+
 def test_munkres_tie_breaking_matches_reference(golden_dir):
     from scd_b200 import naming
     g = np.load(os.path.join(golden_dir, 'hungarian.npz'))

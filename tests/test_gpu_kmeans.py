@@ -348,48 +348,6 @@ def test_host_features_are_assigned_in_panels_under_their_upload():
     assert torch.allclose(norms[:k].cpu(), (cen_o - C).norm(dim=1), atol=1e-5)
 
 
-@pytest.mark.parametrize('n,d,k', [(5000, 768, 100), (127, 256, 7), (128 * 148 * 2 + 77, 512, 160), (40000, 768, 200),
-                                    (9000, 96, 33), (3000, 768, 256)])
-def test_estep_with_fused_mstep_equals_the_two_pass_path(n, d, k):
-    """scd_estep_mstep (one pass over X: argmin, then the tile's rows re-read from L2 and reduced into sums[label]) against
-    the separate E-step + counting sort + segment sum: identical labels / inertia, identical counts, sums to fp32
-    summation order; panel-wise accumulation (SCD_ESTEP_ACCUMULATE) gives the same totals; and the M-step of the oracle."""
-    g = torch.Generator().manual_seed(n + d + k)
-    X = torch.nn.functional.normalize(torch.randn(n, d, generator=g) + 2.0 * torch.randn(k, d, generator=g)[torch.randint(0, k, (n,), generator=g)], dim=1)
-    C = X[torch.randperm(n, generator=g)[:k]].clone()
-    Xd, Cd = X.cuda(), C.cuda()
-    es = kmeans._EStep(k, d, Xd.device)
-    if not es.fusable(n):
-        pytest.skip('no fused plan for this shape')
-    lab2 = torch.empty(n, dtype=torch.int64, device='cuda'); in2 = torch.zeros(1, dtype=torch.float64, device='cuda')
-    ms2 = kmeans._MStep(n, d, k, Xd.device)
-    es.run(Xd, Cd, lab2, in2)
-    ms2.sums_counts(Xd, lab2)
-    lab1 = torch.empty(n, dtype=torch.int64, device='cuda'); in1 = torch.zeros(1, dtype=torch.float64, device='cuda')
-    ms1 = kmeans._MStep(n, d, k, Xd.device)
-    for rep in range(3):                                  # back to back: the sums are zeroed by every launch
-        in1.zero_()
-        es.run(Xd, Cd, lab1, in1, mstep=ms1)
-    assert torch.equal(lab1, lab2) and torch.equal(ms1.counts, ms2.counts)
-    assert abs(float(in1) - float(in2)) <= 1e-9 * max(1.0, float(in2))
-    assert torch.allclose(ms1.sums, ms2.sums, atol=2e-4, rtol=1e-5)
-    want = torch.zeros(k, d, dtype=torch.float64).index_add_(0, lab2.cpu(), X.double())
-    assert torch.allclose(ms1.sums.cpu().double(), want, atol=2e-4, rtol=1e-5)
-    # two panels accumulate into the same totals
-    ms3 = kmeans._MStep(n, d, k, Xd.device)
-    cut = (n // 2 // 128) * 128 + 5 if n > 300 else n // 2
-    lab3 = torch.empty(n, dtype=torch.int64, device='cuda')
-    es.run(Xd[:cut], Cd, lab3[:cut], None, mstep=ms3)
-    es.run(Xd[cut:], Cd, lab3[cut:], None, mstep=ms3, accumulate=True)
-    assert torch.equal(lab3, lab2) and torch.equal(ms3.counts, ms2.counts)
-    assert torch.allclose(ms3.sums, ms2.sums, atol=2e-4, rtol=1e-5)
-    # centres after the divide, against the oracle's M-step
-    c_new = torch.empty(k, d, device='cuda')
-    ms1.finalize(Cd, c_new, shift=False)
-    cen_o = kmeans_oracle.mstep(X, lab2.cpu(), C.clone())
-    assert torch.allclose(c_new.cpu(), cen_o, atol=1e-5, equal_nan=True)
-
-
 def test_kpp_per_draw_agreement_with_the_reference_rule_from_identical_state():
     """The per-DRAW disagreement with the reference's k-means++ rule, measured from identical state (VERDICT r1): for 60
     draws the device path gets exactly the centres the oracle has at that point and the same r, and must pick the same

@@ -13,7 +13,7 @@ for (n, v, d, k, sm) in [(700, 900, 768, 5, False), (20000, 700, 128, 1, False),
     vals, idx, _, _ = naming.name_topk_raw(X, vocab, k, sm)
     torch.cuda.synchronize()
     print('name_topk', (n, v, d, k, sm), int(idx.min()), int(idx.max()))
-# k-means: E-step (both kernel variants), M-step, fused E+M, divide; vote (shared-memory and spill tables)
+# k-means: E-step (both kernel variants), M-step, divide; vote (shared-memory and spill tables)
 for (n, d, k) in [(3000, 768, 100), (2000, 256, 300), (1000, 96, 33)]:
     X = torch.nn.functional.normalize(torch.randn(n, d, generator=g), dim=1).cuda()
     C = X[:k].clone()
@@ -22,11 +22,6 @@ for (n, d, k) in [(3000, 768, 100), (2000, 256, 300), (1000, 96, 33)]:
     es.run(X, C, lab, acc)
     ms.sums_counts(X, lab)
     cn = torch.empty_like(C); ms.finalize(C, cn, estep=es if ms.tc else None, shift=False)
-    if es.fusable(n):
-        ms2 = kmeans._MStep(n, d, k, X.device)
-        es.run(X, C, lab, acc, mstep=ms2)
-        torch.cuda.synchronize()
-        assert torch.allclose(ms2.sums, ms.sums, atol=2e-4)
     idx = torch.randint(0, 500, (n, 5), device='cuda')
     out = naming.vote_device(idx, lab, k, 5, 20)
     out2 = naming.vote_device(idx, None, k, 5, 20, presorted=ms)
