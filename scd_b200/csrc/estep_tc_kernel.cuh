@@ -32,6 +32,7 @@
 #pragma once
 #include "ptx.cuh"
 #include <cuda_bf16.h>
+#include <utility>
 
 namespace scd {
 
@@ -104,27 +105,50 @@ struct EsLayout {
   }
 };
 
-// fp32 centroids -> bf16 hi / lo planes [K, D] + ||c||^2
+// ---- The E-step's centroid operands: bf16 hi / lo planes [K, D] and ||c||^2 [K].  centroid_split_kernel,
+// finalize_centers_kernel and finalize_centers_peer_kernel write them, and SCD_ESTEP_PLANES_READY needs all three to give
+// the same bits: each uses es_store_split, and sums ||c_k||^2 in one block of kEsCentroidThreads threads (thread t
+// accumulates d = t, t + kEsCentroidThreads, .. with fmaf, then block_sum_to_thread0).
+constexpr int kEsCentroidThreads = 256;
+
+__device__ __forceinline__ void es_store_split(float c, __nv_bfloat16* hi, __nv_bfloat16* lo, size_t i) {
+  const __nv_bfloat16 h = __float2bfloat16_rn(c);
+  hi[i] = h;
+  lo[i] = __float2bfloat16_rn(c - __bfloat162float(h));
+}
+
+// block-wide sums of per-thread floats in a fixed order: __shfl_down tree in each warp, then thread 0 adds the warps in
+// order; the totals are left in thread 0's arguments only.  Each value gets its own shared array (block_sum_slot): one
+// [n][32] array instead made ptxas schedule the finalize kernels differently.  At most one call per kernel: the slots are
+// static and there is no barrier after thread 0 reads them, so a second call could overwrite them under that read.
+template <int I> __device__ __forceinline__ float* block_sum_slot() { __shared__ float sh[32]; return sh; }
+template <int... I, typename... F>
+__device__ __forceinline__ void block_sum_to_thread0(std::integer_sequence<int, I...>, F&... v) {
+  for (int off = 16; off > 0; off >>= 1) ((v += __shfl_down_sync(0xffffffffu, v, off)), ...);
+  if ((threadIdx.x & 31) == 0) ((block_sum_slot<I>()[threadIdx.x >> 5] = v), ...);
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    ((v = 0.f), ...);
+    for (int w = 0; w < (blockDim.x + 31) / 32; ++w) ((v += block_sum_slot<I>()[w]), ...);
+  }
+}
+template <typename... F>
+__device__ __forceinline__ void block_sum_to_thread0(F&... v) {
+  block_sum_to_thread0(std::make_integer_sequence<int, sizeof...(F)>{}, v...);
+}
+
+// fp32 centroids -> the operands above
 __global__ void centroid_split_kernel(const float* __restrict__ C, int K, int D, __nv_bfloat16* __restrict__ hi,
                                       __nv_bfloat16* __restrict__ lo, float* __restrict__ cnorm) {
   const int k = blockIdx.x;
   float part = 0.f;
   for (int d = threadIdx.x; d < D; d += blockDim.x) {
     const float c = C[(long long)k * D + d];
-    const __nv_bfloat16 h = __float2bfloat16_rn(c);
-    hi[(long long)k * D + d] = h;
-    lo[(long long)k * D + d] = __float2bfloat16_rn(c - __bfloat162float(h));
+    es_store_split(c, hi, lo, (long long)k * D + d);
     part = fmaf(c, c, part);
   }
-  __shared__ float sh[32];
-  for (int off = 16; off > 0; off >>= 1) part += __shfl_down_sync(0xffffffffu, part, off);
-  if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = part;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    float t = 0.f;
-    for (int w = 0; w < (int)((blockDim.x + 31) / 32); ++w) t += sh[w];
-    cnorm[k] = t;
-  }
+  block_sum_to_thread0(part);
+  if (threadIdx.x == 0) cnorm[k] = part;
 }
 
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }

@@ -13,6 +13,7 @@
 #include <cuda_bf16.h>
 #include <stdint.h>
 #include <math.h>
+#include "estep_tc_kernel.cuh"
 
 namespace scd {
 
@@ -357,8 +358,7 @@ __global__ void segment_sum_generic_kernel(const float* __restrict__ X, const in
 }
 
 // centers = sums / counts (0/0 -> NaN, as torch's mean over zero rows), per-cluster move norm; optionally also the
-// next E-step's operands of the new centres - bf16 hi / lo planes and ||c||^2, exactly what centroid_split_kernel
-// (estep_tc_kernel.cuh) would compute from c_new, same summation order - so the iteration loop needs no split launch.
+// next E-step's operands of the new centres (estep_tc_kernel.cuh), so the iteration loop needs no split launch.
 __global__ void finalize_centers_kernel(const float* __restrict__ sums, const float* __restrict__ counts_f, const int* __restrict__ counts_i,
                                         const float* __restrict__ c_old, float* __restrict__ c_new, float* __restrict__ move_norm,
                                         int K, int D, __nv_bfloat16* __restrict__ plane_hi, __nv_bfloat16* __restrict__ plane_lo,
@@ -371,24 +371,14 @@ __global__ void finalize_centers_kernel(const float* __restrict__ sums, const fl
     c_new[(long long)k * D + d] = c;
     if (c_old) { const float df = c - c_old[(long long)k * D + d]; part += df * df; }
     if (plane_hi) {
-      const __nv_bfloat16 h = __float2bfloat16_rn(c);
-      plane_hi[(long long)k * D + d] = h;
-      plane_lo[(long long)k * D + d] = __float2bfloat16_rn(c - __bfloat162float(h));
+      es_store_split(c, plane_hi, plane_lo, (long long)k * D + d);
       npart = fmaf(c, c, npart);
     }
   }
-  __shared__ float sh[32], shn[32];
-  for (int off = 16; off > 0; off >>= 1) {
-    part += __shfl_down_sync(0xffffffffu, part, off);
-    npart += __shfl_down_sync(0xffffffffu, npart, off);
-  }
-  if ((threadIdx.x & 31) == 0) { sh[threadIdx.x >> 5] = part; shn[threadIdx.x >> 5] = npart; }
-  __syncthreads();
+  block_sum_to_thread0(part, npart);
   if (threadIdx.x == 0) {
-    float t = 0.f, tn = 0.f;
-    for (int w = 0; w < (blockDim.x + 31) / 32; ++w) { t += sh[w]; tn += shn[w]; }
-    if (move_norm) move_norm[k] = sqrtf(t);
-    if (cnorm) cnorm[k] = tn;
+    if (move_norm) move_norm[k] = sqrtf(part);
+    if (cnorm) cnorm[k] = npart;
   }
 }
 

@@ -20,6 +20,7 @@
 // clock and traps with a message instead of hanging the GPU (a rank that died, or ranks launching different sequences).
 #pragma once
 #include "ptx.cuh"
+#include "estep_tc_kernel.cuh"
 #include <cuda_bf16.h>
 
 namespace scd {
@@ -128,7 +129,7 @@ __global__ void peer_barrier_kernel(const PeerPtrs pp, int channel) {
 __host__ __device__ inline size_t peer_mstep_inertia_word(int K, int D) { return (((size_t)K * D + K + 1) / 2) * 2; }
 __host__ __device__ inline size_t peer_mstep_words(int K, int D) { return peer_mstep_inertia_word(K, D) + 2; }
 
-__global__ void __launch_bounds__(256)
+__global__ void __launch_bounds__(kEsCentroidThreads)
 finalize_centers_peer_kernel(const PeerPtrs pp, int channel, size_t buf_word_offset, const float* __restrict__ c_old,
                              float* __restrict__ c_new, float* __restrict__ move_norm, float* __restrict__ counts_out,
                              double* __restrict__ inertia_out, int K, int D, __nv_bfloat16* __restrict__ plane_hi,
@@ -189,30 +190,18 @@ finalize_centers_peer_kernel(const PeerPtrs pp, int channel, size_t buf_word_off
       const float c = s[q] / cnt;                      // 0 / 0 -> NaN row, as torch's mean over zero rows
       c_new[(size_t)k * D + d] = c;
       if (c_old) { const float df = c - c_old[(size_t)k * D + d]; part += df * df; }
-      if (plane_hi) {
-        const __nv_bfloat16 h = __float2bfloat16_rn(c);
-        plane_hi[(size_t)k * D + d] = h;
-        plane_lo[(size_t)k * D + d] = __float2bfloat16_rn(c - __bfloat162float(h));
-      }
+      if (plane_hi) es_store_split(c, plane_hi, plane_lo, (size_t)k * D + d);
     }
   }
-  // ||c||^2 of the next E-step must have centroid_split_kernel's summation order (thread t owns d = t, t + 256, ..): a
-  // second, cheap pass over the row this block has just written
+  // ||c||^2 must be summed in the operands' order (estep_tc_kernel.cuh), not in the 4-wide one above: a second, cheap pass
+  // over the row this block has just written
   __syncthreads();
   if (plane_hi)
     for (int d = threadIdx.x; d < D; d += blockDim.x) { const float c = c_new[(size_t)k * D + d]; npart = fmaf(c, c, npart); }
-  __shared__ float sh[32], shn[32];
-  for (int off = 16; off > 0; off >>= 1) {
-    part += __shfl_down_sync(0xffffffffu, part, off);
-    npart += __shfl_down_sync(0xffffffffu, npart, off);
-  }
-  if ((threadIdx.x & 31) == 0) { sh[threadIdx.x >> 5] = part; shn[threadIdx.x >> 5] = npart; }
-  __syncthreads();
+  block_sum_to_thread0(part, npart);
   if (threadIdx.x == 0) {
-    float t = 0.f, tn = 0.f;
-    for (int w = 0; w < (blockDim.x + 31) / 32; ++w) { t += sh[w]; tn += shn[w]; }
-    if (move_norm) move_norm[k] = sqrtf(t);
-    if (cnorm) cnorm[k] = tn;
+    if (move_norm) move_norm[k] = sqrtf(part);
+    if (cnorm) cnorm[k] = npart;
   }
   peer_finish(pp, channel, target);
 }

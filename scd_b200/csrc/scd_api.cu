@@ -73,6 +73,18 @@ int device_sm_count() {
   return n;
 }
 
+// Raises Kernel's dynamic shared-memory limit on the current device to `bytes` unless it is set that high already.
+template <auto Kernel>
+int allow_dynamic_smem(int bytes) {
+  static int set[kMaxDevices] = {};
+  const int dev = current_device_slot();
+  if (bytes > set[dev]) {
+    SCD_CUDA(cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+    set[dev] = bytes;
+  }
+  return 0;
+}
+
 // ---------------------------------------------------------------- tensor maps
 using EncodeTiledFn = CUresult (*)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                    const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
@@ -136,9 +148,12 @@ struct NamePlan {
   size_t off_val, off_idx, off_max, off_sum, off_scratch, bytes;
 };
 
+// top-k list length the scoring and merge kernels are compiled for, k in 1..8
+inline int list_len(int k) { return k == 1 ? 1 : (k <= 5 ? 5 : 8); }
+
 bool plan_naming(int64_t N, int64_t V, int k, NamePlan* pl) {
   if (k < 1 || k > 8) return false;
-  pl->kt = k == 1 ? 1 : (k <= 5 ? 5 : 8);
+  pl->kt = list_len(k);
   pl->n_row_blocks = (int)((N + 2 * scd::kBlockM - 1) / (2 * scd::kBlockM));
   pl->tiles_total = (int)((V + scd::kTileN - 1) / scd::kTileN);
   pl->work_total = (long long)pl->n_row_blocks * pl->tiles_total;
@@ -180,16 +195,20 @@ bool plan_naming(int64_t N, int64_t V, int k, NamePlan* pl) {
 
 template <int KT>
 int launch_name_topk(const CUtensorMap& mx, const CUtensorMap& mw, const scd::NameParams& p, int n_pairs, cudaStream_t st) {
-  static bool attr_set[kMaxDevices] = {};
   const int smem = scd::NameSmem::total + 1024;
-  const int dev = current_device_slot();
-  if (!attr_set[dev]) {
-    SCD_CUDA(cudaFuncSetAttribute(scd::name_topk_kernel<KT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    attr_set[dev] = true;
-  }
+  if (int e = allow_dynamic_smem<scd::name_topk_kernel<KT>>(smem)) return e;
   scd::name_topk_kernel<KT><<<2 * n_pairs, scd::kNameThreads, smem, st>>>(mx, mw, p);
   SCD_LAUNCH_CHECK("name_topk_kernel");
   return 0;
+}
+
+// topk_merge_kernel for lists of `kmax` = list_len(k) entries; FULL (every subscript a compile-time constant) when k == kmax
+template <typename IdxT, bool PRESCALED, typename... Args>
+void launch_topk_merge(int kmax, int k, int64_t n_rows, cudaStream_t st, const Args&... args) {
+  auto kernel = scd::topk_merge_kernel<IdxT, PRESCALED, 1, true>;
+  if (kmax == 5) kernel = k == 5 ? scd::topk_merge_kernel<IdxT, PRESCALED, 5, true> : scd::topk_merge_kernel<IdxT, PRESCALED, 5, false>;
+  else if (kmax == 8) kernel = k == 8 ? scd::topk_merge_kernel<IdxT, PRESCALED, 8, true> : scd::topk_merge_kernel<IdxT, PRESCALED, 8, false>;
+  kernel<<<(unsigned)((n_rows + 127) / 128), 128, 0, st>>>(args...);
 }
 
 // ---- counting sort of rows by label: workspace carving shared by the M-step and the vote
@@ -207,11 +226,27 @@ struct SortWs {
 };
 constexpr int kMaxSortK = 11264;          // 44 KB of shared-memory counters (+ the static scan scratch stays under 48 KB)
 
+// ---- E-step workspace carving shared by scd_estep and the finalize entry points that leave the next E-step's operands
+// bf16 hi plane [K, D] | bf16 lo plane [K, D] | ||c||^2 [K], each 256-byte aligned; a null workspace carves null pointers
+struct EsWs {
+  __nv_bfloat16* chi = nullptr; __nv_bfloat16* clo = nullptr; float* cnorm = nullptr;
+  size_t plane;                           // bytes from one plane to the next
+  EsWs(void* ws, int K, int D) : plane(plane_bytes(K, D)) {
+    if (!ws) return;
+    uint8_t* w8 = reinterpret_cast<uint8_t*>(ws);
+    chi = reinterpret_cast<__nv_bfloat16*>(w8);
+    clo = reinterpret_cast<__nv_bfloat16*>(w8 + plane);
+    cnorm = reinterpret_cast<float*>(w8 + 2 * plane);
+  }
+  static size_t plane_bytes(int K, int D) { return align_up((size_t)K * D * 2, 256); }
+  static size_t bytes(int K, int D) { return plane_bytes(K, D) * 2 + align_up((size_t)K * sizeof(float), 256) + 256; }
+};
+
 template <typename LabT>
 int sort_rows_by_label(const LabT* labels, long long stride, int64_t N, int K, int32_t* counts_out, const SortWs& w,
                               float* zero_me, size_t n_zero_floats, cudaStream_t st) {
   SCD_CUDA(cudaMemsetAsync(w.acc, 0, sizeof(int) * ((size_t)K + 1), st));          // accumulator + ticket
-  const int blocks = (int)std::max<long long>(1, std::min<long long>((N + scd::kSortThreads - 1) / scd::kSortThreads, 148 * 4));
+  const int blocks = (int)std::max<long long>(1, std::min<long long>((N + scd::kSortThreads - 1) / scd::kSortThreads, device_sm_count() * 4));
   scd::label_hist_scan_kernel<LabT><<<blocks, scd::kSortThreads, sizeof(int) * (size_t)K, st>>>(
       labels, stride, N, K, w.acc, w.ticket, counts_out, w.offsets, w.cursor, reinterpret_cast<float4*>(zero_me),
       (long long)(n_zero_floats / 4));
@@ -231,18 +266,23 @@ int launch_vote(const IdxT* topk_idx, long long idx_stride, int k_used, int64_t 
                        const int* seg_offsets = nullptr, int seg_world = 0, long long seg_per = 0, int32_t* out_rows = nullptr) {
   if (spill && spill_bytes < scd::vote_spill_bytes(N, k_used)) return fail("vote: spill buffer too small (%zu < %zu)", spill_bytes, scd::vote_spill_bytes(N, k_used));
   SCD_CUDA(cudaMemsetAsync(overflow, 0, sizeof(int), st));
-  static bool attr_set[kMaxDevices][3] = {};
-  const int dev = current_device_slot();
-  constexpr int which = SEG ? 2 : (sizeof(IdxT) == 8 ? 0 : 1);
-  if (!attr_set[dev][which]) {
-    SCD_CUDA(cudaFuncSetAttribute(scd::vote_kernel<IdxT, SEG>, cudaFuncAttributeMaxDynamicSharedMemorySize, scd::kVoteSmemBytes));
-    attr_set[dev][which] = true;
-  }
+  if (int e = allow_dynamic_smem<scd::vote_kernel<IdxT, SEG>>(scd::kVoteSmemBytes)) return e;
   scd::vote_kernel<IdxT, SEG><<<K, scd::kVoteThreads, scd::kVoteSmemBytes, st>>>(
       topk_idx, idx_stride, k_used, order, offsets, K, reinterpret_cast<const long long*>(excluded), n_excluded, M,
       reinterpret_cast<long long*>(out_names), out_counts, out_distinct, overflow, reinterpret_cast<int*>(spill),
       seg_offsets, seg_world, seg_per, out_rows);
   SCD_LAUNCH_CHECK("vote_kernel");
+  return 0;
+}
+
+// the checks every vote entry point makes; `who` names the entry point in the error message
+int check_vote_args(const char* who, int64_t N, int K, int k_total, int k_used, int M, const int64_t* excluded, int n_excluded,
+                    const int64_t* out_names, const int32_t* out_counts, const int32_t* out_distinct, const int32_t* overflow) {
+  if (N < 0 || K <= 0 || k_total <= 0 || k_used <= 0 || k_used > k_total || M <= 0) return fail("%s: bad arguments", who);
+  if (N * (int64_t)k_used >= (1ll << 31)) return fail("%s: N * k_used exceeds the 31-bit position range", who);
+  if (K > kMaxSortK) return fail("%s: K=%d too large", who, K);
+  if (!out_names || !out_counts || !out_distinct || !overflow) return fail("%s: null pointer", who);
+  if (n_excluded > 0 && !excluded) return fail("%s: excluded list is null", who);
   return 0;
 }
 
@@ -287,7 +327,7 @@ int scd_estep_uses_tensor_cores(int64_t N, int D, int K) {
 
 size_t scd_estep_workspace_bytes(int K, int D) {
   if (K <= 0 || D <= 0) return 256;
-  return align_up((size_t)K * D * 2, 256) * 2 + align_up((size_t)K * sizeof(float), 256) + 256;
+  return EsWs::bytes(K, D);
 }
 
 int scd_estep(const float* X, int64_t N, int D, const float* C, int K, int64_t* labels, float* mindist, double* inertia_acc,
@@ -308,13 +348,9 @@ int scd_estep(const float* X, int64_t N, int D, const float* C, int K, int64_t* 
     SCD_LAUNCH_CHECK("sqdist_kernel<fused argmin>");
     return 0;
   }
-  uint8_t* w8 = reinterpret_cast<uint8_t*>(ws);
-  const size_t plane = align_up((size_t)K * D * 2, 256);
-  __nv_bfloat16* chi = reinterpret_cast<__nv_bfloat16*>(w8);
-  __nv_bfloat16* clo = reinterpret_cast<__nv_bfloat16*>(w8 + plane);
-  float* cnorm = reinterpret_cast<float*>(w8 + 2 * plane);
+  const EsWs w(ws, K, D);
   if (!(flags & SCD_ESTEP_PLANES_READY)) {      // scd_finalize_centers(estep_ws = ws) already left the planes of C there
-    scd::centroid_split_kernel<<<K, 256, 0, st>>>(C, K, D, chi, clo, cnorm);
+    scd::centroid_split_kernel<<<K, scd::kEsCentroidThreads, 0, st>>>(C, K, D, w.chi, w.clo, w.cnorm);
     SCD_LAUNCH_CHECK("centroid_split_kernel");
   }
 
@@ -325,7 +361,7 @@ int scd_estep(const float* X, int64_t N, int D, const float* C, int K, int64_t* 
   p.n_tile = p.n_ntiles > 1 ? 256 : ((K + 15) / 16) * 16;
   p.num_kb = (D + scd::kEsBK - 1) / scd::kEsBK;
   p.n_row_tiles = (int)((N + scd::kEsBM - 1) / scd::kEsBM);
-  p.cnorm = cnorm;
+  p.cnorm = w.cnorm;
   p.labels = reinterpret_cast<long long*>(labels);
   p.mindist = mindist;
   p.inertia = inertia_acc;
@@ -333,7 +369,7 @@ int scd_estep(const float* X, int64_t N, int D, const float* C, int K, int64_t* 
   CUtensorMap mx, mc;
   if (int e = make_map_2d(&mx, X, (uint64_t)N, (uint64_t)D, scd::kEsBM, scd::kEsBK, CU_TENSOR_MAP_SWIZZLE_128B, true)) return e;
   // hi and lo planes as one 3-D tensor [2][K][D]: a single box brings both k-slabs of a stage
-  if (int e = make_map_planes(&mc, chi, (uint64_t)K, (uint64_t)D, plane, (uint32_t)p.n_tile, scd::kEsBK)) return e;
+  if (int e = make_map_planes(&mc, w.chi, (uint64_t)K, (uint64_t)D, w.plane, (uint32_t)p.n_tile, scd::kEsBK)) return e;
   // shared-memory plan: the centroid ring takes what n_tile needs, the rest goes to fp32 X stages in flight
   p.b_plane = p.n_tile * scd::kEsBK * 2;          // n_tile % 16 == 0 -> a multiple of 1024 (swizzle-atom aligned)
   // converted-operand ring: six stages in the TMEM columns the two accumulators leave free (32 columns per stage, three
@@ -353,13 +389,7 @@ int scd_estep(const float* X, int64_t N, int D, const float* C, int K, int64_t* 
   }
   const int smem = scd::EsLayout(p.x_stages, p.b_plane, tmem_a).total + 1024;
   if (smem > scd::kEsSmemLimit) return fail("scd_estep: shared-memory plan does not fit (%d bytes)", smem);
-  static int attr_smem[kMaxDevices][2] = {};
-  const int dev = current_device_slot();
-  if (smem > attr_smem[dev][tmem_a]) {
-    if (tmem_a) SCD_CUDA(cudaFuncSetAttribute(scd::estep_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    else SCD_CUDA(cudaFuncSetAttribute(scd::estep_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    attr_smem[dev][tmem_a] = smem;
-  }
+  if (int e = tmem_a ? allow_dynamic_smem<scd::estep_tc_kernel<true>>(smem) : allow_dynamic_smem<scd::estep_tc_kernel<false>>(smem)) return e;
   const int grid = std::min(device_sm_count(), p.n_row_tiles);
   if (tmem_a) scd::estep_tc_kernel<true><<<grid, scd::kEsThreads, smem, st>>>(mx, mc, p);
   else scd::estep_tc_kernel<false><<<grid, scd::kEsThreads, smem, st>>>(mx, mc, p);
@@ -422,7 +452,7 @@ int scd_label_histogram(const int64_t* labels, int64_t N, int K, int32_t* counts
   cudaStream_t st = as_stream(stream);
   SCD_CUDA(cudaMemsetAsync(counts, 0, sizeof(int) * (size_t)K, st));
   if (N > 0) {
-    const int blocks = (int)std::min<long long>((N + 255) / 256, 148 * 8);
+    const int blocks = (int)std::min<long long>((N + 255) / 256, device_sm_count() * 8);
     scd::label_hist_kernel<<<blocks, 256, sizeof(int) * (size_t)K, st>>>(reinterpret_cast<const long long*>(labels), N, K, counts);
     SCD_LAUNCH_CHECK("label_hist_kernel");
   }
@@ -480,16 +510,9 @@ int scd_finalize_centers(const float* sums, const int32_t* counts, const float* 
   if (estep_ws && estep_ws_bytes < scd_estep_workspace_bytes(K, D)) return fail("scd_finalize_centers: estep workspace too small");
   cudaStream_t st = as_stream(stream);
   float* norms = (ws && C_old) ? reinterpret_cast<float*>(ws) : nullptr;
-  __nv_bfloat16 *chi = nullptr, *clo = nullptr;
-  float* cnorm = nullptr;
-  if (estep_ws) {                       // same carving as scd_estep
-    uint8_t* w8 = reinterpret_cast<uint8_t*>(estep_ws);
-    const size_t plane = align_up((size_t)K * D * 2, 256);
-    chi = reinterpret_cast<__nv_bfloat16*>(w8);
-    clo = reinterpret_cast<__nv_bfloat16*>(w8 + plane);
-    cnorm = reinterpret_cast<float*>(w8 + 2 * plane);
-  }
-  scd::finalize_centers_kernel<<<K, 256, 0, st>>>(sums, counts_f, counts, C_old, C_new, norms, K, D, chi, clo, cnorm);
+  const EsWs es(estep_ws, K, D);
+  scd::finalize_centers_kernel<<<K, scd::kEsCentroidThreads, 0, st>>>(sums, counts_f, counts, C_old, C_new, norms, K, D, es.chi, es.clo,
+                                                                      es.cnorm);
   SCD_LAUNCH_CHECK("finalize_centers_kernel");
   if (shift) {
     scd::sum_small_kernel<<<1, 1024, 0, st>>>(norms, K, shift);
@@ -518,7 +541,7 @@ int scd_cast_bf16(const float* in, int64_t n, scd_bf16_t* out, scd_stream_t stre
   if (n < 0) return fail("scd_cast_bf16: bad size");
   if (n == 0) return 0;
   if (!in || !out) return fail("scd_cast_bf16: null pointer");
-  const int blocks = (int)std::min<long long>((n + 255) / 256, 148 * 16);
+  const int blocks = (int)std::min<long long>((n + 255) / 256, device_sm_count() * 16);
   scd::cast_f32_to_bf16_kernel<<<blocks, 256, 0, as_stream(stream)>>>(in, n, reinterpret_cast<__nv_bfloat16*>(out));
   SCD_LAUNCH_CHECK("cast_f32_to_bf16_kernel");
   return 0;
@@ -622,18 +645,10 @@ int scd_name_topk(const scd_bf16_t* X, int64_t N, int D, const scd_bf16_t* Wt, i
   if (e) return e;
 
   const bool stats = want_softmax || row_max || row_sumexp;
-  {
-    const dim3 mg((unsigned)((N + 127) / 128));
-    const scd::NameWork mw_{pl.work_total, pl.tiles_total, pl.n_pairs};
-#define SCD_MERGE(KM, FULL)                                                                                                   \
-    scd::topk_merge_kernel<int, false, KM, FULL><<<mg, 128, 0, st>>>(p.part_val, p.part_idx, stats ? p.part_max : nullptr,          \
-        stats ? p.part_sum : nullptr, pl.n_slots * scd::kEpiHalves, N, pl.kt, k, scale, want_softmax ? 1 : 0, idx_offset, vals, \
-        reinterpret_cast<long long*>(idx), row_max, row_sumexp, mw_)
-    if (pl.kt == 1) SCD_MERGE(1, true);
-    else if (pl.kt == 5) { if (k == 5) SCD_MERGE(5, true); else SCD_MERGE(5, false); }
-    else { if (k == 8) SCD_MERGE(8, true); else SCD_MERGE(8, false); }
-#undef SCD_MERGE
-  }
+  launch_topk_merge<int, false>(pl.kt, k, N, st, p.part_val, p.part_idx, stats ? p.part_max : nullptr, stats ? p.part_sum : nullptr,
+                                pl.n_slots * scd::kEpiHalves, N, pl.kt, k, scale, want_softmax ? 1 : 0, idx_offset, vals,
+                                reinterpret_cast<long long*>(idx), row_max, row_sumexp,
+                                scd::NameWork{pl.work_total, pl.tiles_total, pl.n_pairs});
   SCD_LAUNCH_CHECK("topk_merge_kernel");
   return 0;
 }
@@ -644,18 +659,10 @@ int scd_topk_merge(const float* part_vals, const int64_t* part_idx, const float*
   if (N == 0) return 0;
   if (!part_vals || !part_idx || !vals || !idx) return fail("scd_topk_merge: null pointer");
   if (want_softmax && (!part_max || !part_sum)) return fail("scd_topk_merge: softmax needs per-part row_max / row_sumexp");
-  {
-    const dim3 mg((unsigned)((N + 127) / 128));
-    cudaStream_t st = as_stream(stream);
-#define SCD_MERGE(KM, FULL)                                                                                                   \
-    scd::topk_merge_kernel<long long, true, KM, FULL><<<mg, 128, 0, st>>>(part_vals, reinterpret_cast<const long long*>(part_idx),  \
-        want_softmax ? part_max : nullptr, want_softmax ? part_sum : nullptr, parts, N, k, k, scale, want_softmax ? 1 : 0, 0,  \
-        vals, reinterpret_cast<long long*>(idx), nullptr, nullptr, scd::NameWork{0, 1, 0})
-    if (k == 1) SCD_MERGE(1, true);
-    else if (k <= 5) { if (k == 5) SCD_MERGE(5, true); else SCD_MERGE(5, false); }
-    else { if (k == 8) SCD_MERGE(8, true); else SCD_MERGE(8, false); }
-#undef SCD_MERGE
-  }
+  launch_topk_merge<long long, true>(list_len(k), k, N, as_stream(stream), part_vals, reinterpret_cast<const long long*>(part_idx),
+                                     want_softmax ? part_max : nullptr, want_softmax ? part_sum : nullptr, parts, N, k, k, scale,
+                                     want_softmax ? 1 : 0, 0, vals, reinterpret_cast<long long*>(idx), nullptr, nullptr,
+                                     scd::NameWork{0, 1, 0});
   SCD_LAUNCH_CHECK("topk_merge_kernel<shards>");
   return 0;
 }
@@ -670,11 +677,9 @@ size_t scd_vote_spill_bytes(int64_t N, int k_used) { return scd::vote_spill_byte
 int scd_vote(const int64_t* topk_idx, int k_total, int k_used, const int64_t* cluster_of_row, int64_t N, int K,
              const int64_t* excluded, int n_excluded, int M, int64_t* out_names, int32_t* out_counts, int32_t* out_distinct,
              int32_t* out_rows, int32_t* overflow, void* ws, size_t ws_bytes, void* spill, size_t spill_bytes, scd_stream_t stream) {
-  if (N < 0 || K <= 0 || k_total <= 0 || k_used <= 0 || k_used > k_total || M <= 0) return fail("scd_vote: bad arguments");
-  if (N * (int64_t)k_used >= (1ll << 31)) return fail("scd_vote: N * k_used exceeds the 31-bit position range");
-  if (K > kMaxSortK) return fail("scd_vote: K=%d too large", K);
-  if (!topk_idx || !cluster_of_row || !out_names || !out_counts || !out_distinct || !out_rows || !overflow || !ws) return fail("scd_vote: null pointer");
-  if (n_excluded > 0 && !excluded) return fail("scd_vote: excluded list is null");
+  if (int e = check_vote_args("scd_vote", N, K, k_total, k_used, M, excluded, n_excluded, out_names, out_counts, out_distinct,
+                              overflow)) return e;
+  if (!topk_idx || !cluster_of_row || !out_rows || !ws) return fail("scd_vote: null pointer");
   if (ws_bytes < scd_vote_workspace_bytes(N, K)) return fail("scd_vote: workspace too small");
   cudaStream_t st = as_stream(stream);
   int* counts = reinterpret_cast<int*>(ws);
@@ -687,10 +692,9 @@ int scd_vote(const int64_t* topk_idx, int k_total, int k_used, const int64_t* cl
 int scd_vote_presorted(const int64_t* topk_idx, int k_total, int k_used, const void* mstep_ws, int64_t N, int K,
                        const int64_t* excluded, int n_excluded, int M, int64_t* out_names, int32_t* out_counts,
                        int32_t* out_distinct, int32_t* overflow, void* spill, size_t spill_bytes, scd_stream_t stream) {
-  if (N < 0 || K <= 0 || k_total <= 0 || k_used <= 0 || k_used > k_total || M <= 0) return fail("scd_vote_presorted: bad arguments");
-  if (N * (int64_t)k_used >= (1ll << 31)) return fail("scd_vote_presorted: N * k_used exceeds the 31-bit position range");
-  if (!topk_idx || !mstep_ws || !out_names || !out_counts || !out_distinct || !overflow) return fail("scd_vote_presorted: null pointer");
-  if (n_excluded > 0 && !excluded) return fail("scd_vote_presorted: excluded list is null");
+  if (int e = check_vote_args("scd_vote_presorted", N, K, k_total, k_used, M, excluded, n_excluded, out_names, out_counts, out_distinct,
+                              overflow)) return e;
+  if (!topk_idx || !mstep_ws) return fail("scd_vote_presorted: null pointer");
   const SortWs w(const_cast<void*>(mstep_ws), K);         // as written by scd_mstep_sums
   return launch_vote<long long>(reinterpret_cast<const long long*>(topk_idx), k_total, k_used, N, w.order, w.offsets, K, excluded, n_excluded,
                                 M, out_names, out_counts, out_distinct, overflow, spill, spill_bytes, as_stream(stream));
@@ -702,7 +706,7 @@ int scd_pack_vote_records(const int64_t* labels, const int64_t* topk_idx, int k_
   if (n == 0) return 0;
   if (!labels || !topk_idx || !rec) return fail("scd_pack_vote_records: null pointer");
   if (k_used > 8) return fail("scd_pack_vote_records: k_used=%d unsupported (<= 8)", k_used);
-  const int blocks = (int)std::min<long long>((n + 255) / 256, 148 * 8);
+  const int blocks = (int)std::min<long long>((n + 255) / 256, device_sm_count() * 8);
   scd::pack_vote_records_kernel<<<blocks, 256, 0, as_stream(stream)>>>(reinterpret_cast<const long long*>(labels),
                                                                        reinterpret_cast<const long long*>(topk_idx), k_total, k_used, n, rec);
   SCD_LAUNCH_CHECK("pack_vote_records_kernel");
@@ -712,11 +716,9 @@ int scd_pack_vote_records(const int64_t* labels, const int64_t* topk_idx, int k_
 int scd_vote_records(const int32_t* rec, int k_used, int64_t N, int K, const int64_t* excluded, int n_excluded, int M,
                      int64_t* out_names, int32_t* out_counts, int32_t* out_distinct, int32_t* out_rows, int32_t* overflow,
                      void* ws, size_t ws_bytes, void* spill, size_t spill_bytes, scd_stream_t stream) {
-  if (N < 0 || K <= 0 || k_used <= 0 || M <= 0) return fail("scd_vote_records: bad arguments");
-  if (N * (int64_t)k_used >= (1ll << 31)) return fail("scd_vote_records: N * k_used exceeds the 31-bit position range");
-  if (K > kMaxSortK) return fail("scd_vote_records: K=%d too large", K);
-  if (!rec || !out_names || !out_counts || !out_distinct || !out_rows || !overflow || !ws) return fail("scd_vote_records: null pointer");
-  if (n_excluded > 0 && !excluded) return fail("scd_vote_records: excluded list is null");
+  if (int e = check_vote_args("scd_vote_records", N, K, k_used, k_used, M, excluded, n_excluded, out_names, out_counts, out_distinct,
+                              overflow)) return e;
+  if (!rec || !out_rows || !ws) return fail("scd_vote_records: null pointer");
   if (ws_bytes < scd_vote_workspace_bytes(N, K)) return fail("scd_vote_records: workspace too small");
   cudaStream_t st = as_stream(stream);
   int* counts = reinterpret_cast<int*>(ws);
@@ -752,17 +754,9 @@ int scd_finalize_centers_peer(void* const* peer_bufs, void* const* peer_flags, i
   if (estep_ws && estep_ws_bytes < scd_estep_workspace_bytes(K, D)) return fail("scd_finalize_centers_peer: estep workspace too small");
   scd::PeerPtrs pp;
   if (int e = make_peer_ptrs(&pp, peer_bufs, peer_flags, world, rank, "scd_finalize_centers_peer")) return e;
-  __nv_bfloat16 *chi = nullptr, *clo = nullptr;
-  float* cnorm = nullptr;
-  if (estep_ws) {                       // same carving as scd_estep
-    uint8_t* w8 = reinterpret_cast<uint8_t*>(estep_ws);
-    const size_t plane = align_up((size_t)K * D * 2, 256);
-    chi = reinterpret_cast<__nv_bfloat16*>(w8);
-    clo = reinterpret_cast<__nv_bfloat16*>(w8 + plane);
-    cnorm = reinterpret_cast<float*>(w8 + 2 * plane);
-  }
-  scd::finalize_centers_peer_kernel<<<K, 256, 0, as_stream(stream)>>>(pp, channel, buf_byte_offset / sizeof(float), C_old, C_new,
-                                                                      move_norms, counts_out, inertia_out, K, D, chi, clo, cnorm);
+  const EsWs es(estep_ws, K, D);
+  scd::finalize_centers_peer_kernel<<<K, scd::kEsCentroidThreads, 0, as_stream(stream)>>>(
+      pp, channel, buf_byte_offset / sizeof(float), C_old, C_new, move_norms, counts_out, inertia_out, K, D, es.chi, es.clo, es.cnorm);
   SCD_LAUNCH_CHECK("finalize_centers_peer_kernel");
   return 0;
 }
@@ -776,7 +770,7 @@ int scd_pack_vote_records_peer(void* const* peer_bufs, int world, int rank, size
   if (n == 0) return 0;
   if (!labels || !topk_idx) return fail("scd_pack_vote_records_peer: null pointer");
   if (k_used > 8) return fail("scd_pack_vote_records_peer: k_used=%d unsupported (<= 8)", k_used);
-  const int blocks = (int)std::min<long long>((n + scd::kPackRows - 1) / scd::kPackRows, 148 * 8);
+  const int blocks = (int)std::min<long long>((n + scd::kPackRows - 1) / scd::kPackRows, device_sm_count() * 8);
   scd::pack_vote_records_peer_kernel<<<blocks, 256, 0, as_stream(stream)>>>(pp, buf_byte_offset, reinterpret_cast<const long long*>(labels),
                                                                             reinterpret_cast<const long long*>(topk_idx), k_total, k_used, n, row_offset);
   SCD_LAUNCH_CHECK("pack_vote_records_peer_kernel");
@@ -793,7 +787,7 @@ int scd_pack_sorted_records_peer(void* const* peer_bufs, int world, int rank, si
   scd::PeerPtrs pp;
   if (int e = make_peer_ptrs(&pp, peer_bufs, nullptr, world, rank, "scd_pack_sorted_records_peer")) return e;
   const SortWs w(const_cast<void*>(mstep_ws), K);           // as written by scd_mstep_sums on this rank's labels
-  const int blocks = (int)std::max<long long>(1, std::min<long long>((n + scd::kPackRows - 1) / scd::kPackRows, 148 * 8));
+  const int blocks = (int)std::max<long long>(1, std::min<long long>((n + scd::kPackRows - 1) / scd::kPackRows, device_sm_count() * 8));
   scd::pack_sorted_records_peer_kernel<<<blocks, 256, 0, as_stream(stream)>>>(pp, rec_byte_offset, off_byte_offset,
       reinterpret_cast<const long long*>(topk_idx), k_total, k_used, n, row_offset, w.order, w.offsets, K);
   SCD_LAUNCH_CHECK("pack_sorted_records_peer_kernel");
@@ -804,14 +798,12 @@ int scd_vote_segments(const int32_t* rec, int k_used, int64_t n_total, int64_t p
                       const int64_t* excluded, int n_excluded, int M, int64_t* out_names, int32_t* out_counts,
                       int32_t* out_distinct, int32_t* out_rows, int32_t* overflow, void* spill, size_t spill_bytes,
                       scd_stream_t stream) {
-  if (per < 0 || world < 1 || world > scd::kVoteMaxSeg || K <= 0 || k_used <= 0 || M <= 0 || n_total < 0 || n_total > per * world)
-    return fail("scd_vote_segments: bad arguments");
-  const int64_t N = n_total;
-  if (N * (int64_t)k_used >= (1ll << 31)) return fail("scd_vote_segments: N * k_used exceeds the 31-bit position range");
-  if (!rec || !seg_offsets || !out_names || !out_counts || !out_distinct || !out_rows || !overflow) return fail("scd_vote_segments: null pointer");
-  if (n_excluded > 0 && !excluded) return fail("scd_vote_segments: excluded list is null");
-  return launch_vote<int, true>(rec, 1 + k_used, k_used, N, nullptr, nullptr, K, excluded, n_excluded, M, out_names, out_counts, out_distinct,
-                                overflow, spill, spill_bytes, as_stream(stream), seg_offsets, world, per, out_rows);
+  if (per < 0 || world < 1 || world > scd::kVoteMaxSeg || n_total > per * world) return fail("scd_vote_segments: bad arguments");
+  if (int e = check_vote_args("scd_vote_segments", n_total, K, k_used, k_used, M, excluded, n_excluded, out_names, out_counts,
+                              out_distinct, overflow)) return e;
+  if (!rec || !seg_offsets || !out_rows) return fail("scd_vote_segments: null pointer");
+  return launch_vote<int, true>(rec, 1 + k_used, k_used, n_total, nullptr, nullptr, K, excluded, n_excluded, M, out_names, out_counts,
+                                out_distinct, overflow, spill, spill_bytes, as_stream(stream), seg_offsets, world, per, out_rows);
 }
 
 int scd_contingency(const void* y_pred, int pred_is_f64, const void* y_true, int true_is_f64, int64_t N, int D,

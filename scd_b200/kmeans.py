@@ -96,7 +96,6 @@ class _MStep:
         self.counts_f = self.packed[k * d:k * d + k]
         self.counts = torch.empty(k, dtype=torch.int32, device=device)
         self.peer = None                                  # (PeerExchange, block) while the sums live in a peer-mapped block
-        self.sorted_for = None                            # data_ptr of the labels whose counting sort is in `ws` (vote reuse)
         self.norms = torch.zeros(max(k, 1), dtype=torch.float32, device=device)     # ||c_new[k] - c_old[k]||
         self.shift = torch.zeros(1, dtype=torch.float32, device=device)
         self.tc = bool(lib.scd_estep_uses_tensor_cores(max(n, 1), d, k))
@@ -110,7 +109,6 @@ class _MStep:
         lib = _lib.load()
         _lib.check(lib.scd_mstep_sums(X.data_ptr(), labels.data_ptr(), self.n, self.d, self.k, self.sums.data_ptr(),
                                       self.counts.data_ptr(), self.ws.data_ptr(), self.ws.numel(), _stream()), 'scd_mstep_sums')
-        self.sorted_for = labels.data_ptr()
 
     def finalize_peer(self, c_old, c_new, inertia_out, estep: '_EStep | None' = None):
         """The row-sharded M-step's all-reduce + divide in one launch over peer memory (``scd_finalize_centers_peer``);

@@ -249,6 +249,23 @@ class VotePlan:
         return (_lib.ptr(self.spill), 0 if self.spill is None else self.spill.numel())
 
 
+def _vote_plan(plan, n: int, K: int, M: int, k_used: int, device, n_at_least: bool = False) -> VotePlan:
+    """``plan`` checked against the vote's shape (``n_at_least``: any ``plan.n >= n``), or a new one when it is None."""
+    if plan is None:
+        return VotePlan(n, K, M, device, k_used=k_used)
+    if (plan.K, plan.M) != (K, M) or plan.k_used < k_used or (plan.n < n if n_at_least else plan.n != n):
+        raise ValueError('VotePlan was built for a different shape')
+    return plan
+
+
+def _excluded(known_name_idx, device):
+    """``(int64 device tensor, count)`` of the names the vote skips; ``(None, 0)`` when there are none."""
+    if known_name_idx is None or not len(known_name_idx):
+        return None, 0
+    excl = torch.as_tensor(np.asarray(list(known_name_idx), dtype=np.int64), device=device)
+    return excl, int(excl.numel())
+
+
 def vote_device(name_idx_topk: torch.Tensor, cluster_of_row, n_clusters: int, top_k: int, num_common: int,
                 known_name_idx=None, plan: VotePlan | None = None, presorted=None):
     """Device vote: per cluster the ``num_common`` most common names of ``name_idx_topk[rows, :top_k]``
@@ -264,29 +281,22 @@ def vote_device(name_idx_topk: torch.Tensor, cluster_of_row, n_clusters: int, to
     n, kt = int(idx.shape[0]), int(idx.shape[1])
     dev = idx.device
     K, M = int(n_clusters), int(num_common)
-    if plan is None:
-        plan = VotePlan(n, K, M, dev, k_used=int(top_k))
-    elif (plan.n, plan.K, plan.M) != (n, K, M) or plan.k_used < int(top_k):
-        raise ValueError('VotePlan was built for a different shape')
-    excl = None
-    if known_name_idx is not None and len(known_name_idx):
-        excl = torch.as_tensor(np.asarray(list(known_name_idx), dtype=np.int64), device=dev)
+    plan = _vote_plan(plan, n, K, M, int(top_k), dev)
+    excl, n_excl = _excluded(known_name_idx, dev)
     lib = _lib.load()
     if presorted is not None:
         if (presorted.n, presorted.k) != (n, K):
             raise ValueError('presorted M-step does not match the vote shape')
-        _lib.check(lib.scd_vote_presorted(idx.data_ptr(), kt, int(top_k), presorted.ws.data_ptr(), n, K, _lib.ptr(excl),
-                                          0 if excl is None else int(excl.numel()), M, plan.names.data_ptr(),
-                                          plan.counts.data_ptr(), plan.distinct.data_ptr(), plan.overflow.data_ptr(),
-                                          *plan.spill_args(), _stream()), 'scd_vote_presorted')
+        _lib.check(lib.scd_vote_presorted(idx.data_ptr(), kt, int(top_k), presorted.ws.data_ptr(), n, K, _lib.ptr(excl), n_excl, M,
+                                          plan.names.data_ptr(), plan.counts.data_ptr(), plan.distinct.data_ptr(),
+                                          plan.overflow.data_ptr(), *plan.spill_args(), _stream()), 'scd_vote_presorted')
         return plan.names, plan.counts, plan.distinct, presorted.counts, plan.overflow
     cl = cluster_of_row
     if not (torch.is_tensor(cl) and cl.is_cuda and cl.dtype == torch.int64 and cl.is_contiguous()):
         cl = torch.as_tensor(cl).to('cuda').to(torch.int64).contiguous()
-    _lib.check(lib.scd_vote(idx.data_ptr(), kt, int(top_k), cl.data_ptr(), n, K, _lib.ptr(excl),
-                            0 if excl is None else int(excl.numel()), M, plan.names.data_ptr(), plan.counts.data_ptr(),
-                            plan.distinct.data_ptr(), plan.rows.data_ptr(), plan.overflow.data_ptr(), plan.ws.data_ptr(),
-                            plan.ws.numel(), *plan.spill_args(), _stream()), 'scd_vote')
+    _lib.check(lib.scd_vote(idx.data_ptr(), kt, int(top_k), cl.data_ptr(), n, K, _lib.ptr(excl), n_excl, M, plan.names.data_ptr(),
+                            plan.counts.data_ptr(), plan.distinct.data_ptr(), plan.rows.data_ptr(), plan.overflow.data_ptr(),
+                            plan.ws.data_ptr(), plan.ws.numel(), *plan.spill_args(), _stream()), 'scd_vote')
     return plan.names, plan.counts, plan.distinct, plan.rows, plan.overflow
 
 
@@ -306,15 +316,10 @@ def vote_records(records: torch.Tensor, n_clusters: int, num_common: int, known_
     """The vote over gathered ``[N, 1 + top_k]`` int32 records (see ``pack_vote_records``); same outputs as ``vote_device``."""
     n, top_k = int(records.shape[0]), int(records.shape[1]) - 1
     K, M = int(n_clusters), int(num_common)
-    if plan is None:
-        plan = VotePlan(n, K, M, records.device, k_used=top_k)
-    elif (plan.n, plan.K, plan.M) != (n, K, M) or plan.k_used < top_k:
-        raise ValueError('VotePlan was built for a different shape')
-    excl = None
-    if known_name_idx is not None and len(known_name_idx):
-        excl = torch.as_tensor(np.asarray(list(known_name_idx), dtype=np.int64), device=records.device)
+    plan = _vote_plan(plan, n, K, M, top_k, records.device)
+    excl, n_excl = _excluded(known_name_idx, records.device)
     lib = _lib.load()
-    _lib.check(lib.scd_vote_records(records.data_ptr(), top_k, n, K, _lib.ptr(excl), 0 if excl is None else int(excl.numel()), M,
+    _lib.check(lib.scd_vote_records(records.data_ptr(), top_k, n, K, _lib.ptr(excl), n_excl, M,
                                     plan.names.data_ptr(), plan.counts.data_ptr(), plan.distinct.data_ptr(), plan.rows.data_ptr(),
                                     plan.overflow.data_ptr(), plan.ws.data_ptr(), plan.ws.numel(), *plan.spill_args(), _stream()),
                'scd_vote_records')
@@ -330,16 +335,11 @@ def vote_segments(records: torch.Tensor, seg_offsets: torch.Tensor, n_clusters: 
     top_k = int(records.shape[1]) - 1
     K, M = int(n_clusters), int(num_common)
     n_total = world * per if n_total is None else int(n_total)
-    if plan is None:
-        plan = VotePlan(n_total, K, M, records.device, k_used=top_k)
-    elif (plan.K, plan.M) != (K, M) or plan.k_used < top_k or plan.n < n_total:
-        raise ValueError('VotePlan was built for a different shape')
-    excl = None
-    if known_name_idx is not None and len(known_name_idx):
-        excl = torch.as_tensor(np.asarray(list(known_name_idx), dtype=np.int64), device=records.device)
+    plan = _vote_plan(plan, n_total, K, M, top_k, records.device, n_at_least=True)
+    excl, n_excl = _excluded(known_name_idx, records.device)
     lib = _lib.load()
     _lib.check(lib.scd_vote_segments(records.data_ptr(), top_k, n_total, per, world, seg_offsets.data_ptr(), K, _lib.ptr(excl),
-                                     0 if excl is None else int(excl.numel()), M, plan.names.data_ptr(), plan.counts.data_ptr(),
+                                     n_excl, M, plan.names.data_ptr(), plan.counts.data_ptr(),
                                      plan.distinct.data_ptr(), plan.rows.data_ptr(), plan.overflow.data_ptr(), *plan.spill_args(), _stream()),
                'scd_vote_segments')
     return plan.names, plan.counts, plan.distinct, plan.rows, plan.overflow

@@ -70,8 +70,9 @@ def test_estep_many_centroid_tiles_against_oracle(k, d):
 
 
 def test_finalize_leaves_the_next_esteps_operands():
-    """scd_finalize_centers(estep_ws=...) + SCD_ESTEP_PLANES_READY gives bit-identical labels / distances to the E-step
-    that splits the centres itself - including a NaN centre (empty cluster)."""
+    """scd_finalize_centers(estep_ws=...) leaves the same workspace bytes (hi / lo planes, ||c||^2) as the E-step's own
+    split of the new centres, and with SCD_ESTEP_PLANES_READY gives bit-identical labels / distances - including a NaN
+    centre (empty cluster)."""
     cfg = synth.Config('t', 20000, 100, 10, 11)
     data = synth.make(cfg, d=768)
     X, C0 = data['X'].cuda(), data['C0'].cuda()
@@ -84,6 +85,7 @@ def test_finalize_leaves_the_next_esteps_operands():
     c_new = torch.empty_like(C0)
     ms.finalize(C0, c_new, estep=es, shift=False)
     assert es.ready_for == c_new.data_ptr() and torch.isnan(c_new[7]).all()
+    ws_finalize = es.ws.clone()
     l1, m1 = torch.empty_like(labels), torch.empty(n, device='cuda')
     es.run(X, c_new, l1, None, m1)                            # uses the operands finalize left behind
     assert es.ready_for is None
@@ -91,6 +93,9 @@ def test_finalize_leaves_the_next_esteps_operands():
     kmeans._estep(X, c_new, l2, None, m2)                     # splits c_new itself
     assert torch.equal(l1, l2) and torch.equal(m1.isnan(), m2.isnan()) and torch.equal(m1[~m1.isnan()], m2[~m2.isnan()])
     assert (l1 == 7).all()                                    # torch.min: a NaN distance beats any number
+    es.ready_for = None
+    es.run(X, c_new, l2, None)                                # centroid_split_kernel rewrites es.ws from c_new
+    assert torch.equal(es.ws, ws_finalize)                    # byte for byte, the NaN row of cluster 7 included
     # the host-side sum of the move norms is the device-side shift
     ms.finalize(C0, c_new)
     assert torch.equal(torch.isnan(ms.shift), torch.isnan(ms.norms[:k].sum().view(1)))
