@@ -66,16 +66,14 @@ def test_pairwise_distance_matches_golden(golden_dir):
 
 
 def test_estep_tie_and_nan_rules():
-    # duplicate centroids: ties go to the lowest index; a NaN centroid wins every row (torch.min semantics)
-    X = synth.unit_rows(torch.randn(300, 32, generator=torch.Generator().manual_seed(1)))
-    C = X[:6].clone(); C[4] = C[1]; C[5] = C[0]
-    lab = kmeans.predict(X.cuda(), C.cuda()).cpu()
-    want = kmeans_oracle.pairwise_distance(X, C, None).argmin(dim=1)
-    assert torch.equal(lab, want) and not ((lab == 4) | (lab == 5)).any()
-    C[3] = float('nan')
-    lab = kmeans.predict(X.cuda(), C.cuda()).cpu()
-    assert torch.equal(lab, torch.min(kmeans_oracle.pairwise_distance(X, C, None), dim=1)[1])
-    assert (lab == 3).all()
+    """The fp32 direct-form E-step (D = 32 / 36: the tensor-core path needs D % 8 == 0 and D >= 40) on exact-grid data:
+    duplicate centroids tie to the lowest index, a NaN centroid wins every row (torch.min), the first of two NaNs wins,
+    a NaN in a row of X gives label 0 - labels, distances and inertia equal the fp64 reference bit for bit
+    (test_gpu_exact_grid.py runs the same cases on the tensor-core kernel)."""
+    from test_gpu_exact_grid import check_estep_grid
+    for d in (32, 36):
+        for k in (12, 161, 257, 1024):
+            check_estep_grid(k, d)
 
 
 @pytest.mark.parametrize('n,d,k', [(600, 64, 12), (5000, 768, 100), (257, 4, 3), (3000, 100, 1000), (1, 8, 2)])

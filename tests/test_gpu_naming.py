@@ -11,7 +11,7 @@ import pytest
 import torch
 
 from oracle import naming_oracle
-from scd_b200 import naming, synth
+from scd_b200 import kmeans, naming, synth
 
 pytestmark = pytest.mark.gpu
 TAU = 1e-3
@@ -125,6 +125,17 @@ def test_vote_matches_oracle_counters(known):
     names, counts, distinct, rows, ovf = naming.vote_device(idx.cuda(), preds, k, 5, 20, known)
     assert int(ovf) == 0 and torch.equal(rows.cpu().long(), torch.bincount(torch.from_numpy(preds), minlength=k))
     assert [int(x) for x in distinct.cpu()] == [len(co_c) for co_c in naming_oracle.vote(idx, preds, list(range(k)), 5, known_name_idx=known).values()]
+    # the same vote on the label sort the M-step has just made (scd_vote_presorted): that sort is not stable, the vote's
+    # first-occurrence tie order must not depend on it
+    ms = kmeans._MStep(n, 4, k, 'cuda')
+    ms.sums_counts(torch.randn(n, 4, generator=torch.Generator().manual_seed(4)).cuda(), torch.from_numpy(preds).cuda())
+    for top_k in (5, 2):
+        co = naming_oracle.vote(idx, preds, list(range(k)), top_k, known_name_idx=known)
+        names, counts, distinct, rows, ovf = naming.vote_device(idx.cuda(), None, k, top_k, 20, known, presorted=ms)
+        assert int(ovf) == 0 and torch.equal(rows.cpu().long(), torch.bincount(torch.from_numpy(preds), minlength=k))
+        for c in range(k):
+            assert [(int(a), int(b)) for a, b in zip(names[c].tolist(), counts[c].tolist()) if a >= 0] == _counter_list(co[c]), c
+            assert int(distinct[c]) == len(co[c])
 
 
 def test_unsup_voting_loop_matches_reference_golden(golden_dir):

@@ -235,16 +235,23 @@ def test_vote_clusters_beyond_the_shared_memory_table(known):
     preds[:5] = 2
     idx = torch.randint(0, v, (n, 5), generator=g)
     idx[:, 0] = torch.randint(0, 50, (n,), generator=g)
-    names, counts, distinct, rows, ovf = naming.vote_device(idx.cuda(), preds.cuda(), k, 5, 20, known)
-    assert int(ovf.item()) == 0 and int(distinct.min()) > 16384
+    # also on the label sort the M-step has just made (scd_vote_presorted): that sort is not stable, the vote's
+    # first-occurrence tie order must not depend on it
+    ms = kmeans._MStep(n, 4, k, 'cuda')
+    ms.sums_counts(torch.randn(n, 4, generator=torch.Generator().manual_seed(14)).cuda(), preds.cuda())
     co = naming_oracle.vote(idx, preds.numpy(), list(range(k)), 5, known_name_idx=known)
-    for c in range(k):
-        want = [(int(a), int(b)) for a, b in co[c].most_common(20)]
-        got = [(int(a), int(b)) for a, b in zip(names[c].tolist(), counts[c].tolist()) if a >= 0]
-        assert got == want
-        assert int(distinct[c]) == len(co[c])
+    for presorted in (None, ms):
+        names, counts, distinct, rows, ovf = naming.vote_device(idx.cuda(), preds.cuda(), k, 5, 20, known, presorted=presorted)
+        assert int(ovf.item()) == 0 and int(distinct.min()) > 16384
+        assert torch.equal(rows.cpu().long(), torch.bincount(preds, minlength=k))
+        for c in range(k):
+            want = [(int(a), int(b)) for a, b in co[c].most_common(20)]
+            got = [(int(a), int(b)) for a, b in zip(names[c].tolist(), counts[c].tolist()) if a >= 0]
+            assert got == want
+            assert int(distinct[c]) == len(co[c])
     # top_k = 2 of the same lists, and many ties at the selection threshold (every name seen once or twice)
     idx2 = torch.randperm(n * 5, generator=g).view(n, 5) % 200_000
-    names, counts, _, _, ovf = naming.vote_device(idx2.cuda(), preds.cuda(), k, 2, 20)
-    assert int(ovf.item()) == 0
-    _check_vote(names, counts, idx2, preds.numpy(), list(range(k)), 2, 20)
+    for presorted in (None, ms):
+        names, counts, _, _, ovf = naming.vote_device(idx2.cuda(), preds.cuda(), k, 2, 20, presorted=presorted)
+        assert int(ovf.item()) == 0
+        _check_vote(names, counts, idx2, preds.numpy(), list(range(k)), 2, 20)
