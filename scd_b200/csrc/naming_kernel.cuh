@@ -387,9 +387,10 @@ name_topk_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
               if (t == 0 && !te_after_token) { const long long c0 = prof ? clock64() : 0;
                 ptx::mbar_wait_nocall(a_full_bar(kb), my_item_no & 1, 400 + kb);
                 if (prof) pf_a += clock64() - c0; }
+              // both stages in one probe (their barrier round trips overlap).  Neither can complete a later phase
+              // meanwhile: their next fills wait for the releases this k-block's MMAs commit.
               { const long long c0 = prof ? clock64() : 0;
-                ptx::mbar_wait_nocall(full_bar(stage0), phase0, 500 + stage0);
-                ptx::mbar_wait_nocall(full_bar(stage1), phase1, 500 + stage1);
+                ptx::mbar_wait2_nocall(full_bar(stage0), phase0, full_bar(stage1), phase1, 500 + stage0);
                 if (prof) pf_b += clock64() - c0; }
               ptx::tc_fence_after_sync();
               const long long tr0 = trace ? clock64() : 0;

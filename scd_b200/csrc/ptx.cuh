@@ -114,16 +114,16 @@ __device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
 }
 // Two barriers probed by one statement: both try_waits are in flight before either predicate is read, so
 // the ~100-cycle barrier round trips overlap (a single-thread issue loop pays the latency once per pair).
-__device__ __forceinline__ bool mbar_try_wait2(uint32_t bar0, uint32_t bar1, uint32_t parity) {
+__device__ __forceinline__ bool mbar_try_wait2(uint32_t bar0, uint32_t parity0, uint32_t bar1, uint32_t parity1) {
   uint32_t ok;
   asm volatile(
       "{\n\t.reg .pred p, q;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %3;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 q, [%2], %3;\n\t"
+      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
+      "mbarrier.try_wait.parity.shared::cta.b64 q, [%3], %4;\n\t"
       "and.pred p, p, q;\n\t"
       "selp.u32 %0, 1, 0, p;\n\t}"
       : "=r"(ok)
-      : "r"(bar0), "r"(bar1), "r"(parity)
+      : "r"(bar0), "r"(parity0), "r"(bar1), "r"(parity1)
       : "memory");
   return ok != 0;
 }
@@ -184,11 +184,17 @@ __device__ __forceinline__ void mbar_wait_nocall(uint32_t bar, uint32_t parity, 
   }
 }
 
-__device__ __forceinline__ void mbar_wait2(uint32_t bar0, uint32_t bar1, uint32_t parity, int tag = 0) {
-  if (mbar_try_wait2(bar0, bar1, parity)) return;
+// Both barriers of mbar_try_wait2, bounded like mbar_wait_nocall.  Sound only if neither barrier can complete a further
+// phase while the waiter spins (each is released by the waiter's own later work).
+__device__ __forceinline__ void mbar_wait2_nocall(uint32_t bar0, uint32_t parity0, uint32_t bar1, uint32_t parity1, int tag = 0) {
+  if (mbar_try_wait2(bar0, parity0, bar1, parity1)) return;
   WaitClock clk;
-  while (!mbar_try_wait2(bar0, bar1, parity)) {
-    if (clk.expired()) mbar_timeout_trap(bar0, parity, tag);
+  while (!mbar_try_wait2(bar0, parity0, bar1, parity1)) {
+    if (clk.expired()) {
+      *reinterpret_cast<volatile int*>(&g_mbar_timeout_tag) = tag;
+      __threadfence();
+      __trap();
+    }
   }
 }
 
