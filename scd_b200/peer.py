@@ -45,29 +45,47 @@ class PeerExchange:
     def __init__(self, group, k: int, d: int, n_total: int = 0, k_used: int = 0, device=None):
         import torch.distributed as dist
         import torch.distributed._symmetric_memory as symm_mem
-        lib = _lib.load()
         self.group = group if group is not None else dist.group.WORLD
-        self.world, self.rank = dist.get_world_size(self.group), dist.get_rank(self.group)
+        self.world = dist.get_world_size(self.group)
         if self.world > 16:
             raise ValueError('PeerExchange supports up to 16 ranks of one NVLink domain')
-        self.k, self.d, self.n_total, self.k_used = int(k), int(d), int(n_total), int(k_used)
         dev = torch.device('cuda', torch.cuda.current_device()) if device is None else torch.device(device)
-        flag_bytes = _align(lib.scd_peer_flag_bytes())
+        buf = symm_mem.empty(self.buffer_bytes(self.world, k, d, n_total, k_used), dtype=torch.uint8, device=dev)
+        buf.zero_()
+        self.handle = symm_mem.rendezvous(buf, self.group.group_name)
+        torch.cuda.synchronize(dev)
+        dist.barrier(group=self.group)                      # every pad is zero before anybody signals
+        self._carve(self.world, dist.get_rank(self.group), k, d, n_total, k_used, buf, [int(p) for p in self.handle.buffer_ptrs])
+
+    @classmethod
+    def buffer_bytes(cls, world: int, k: int, d: int, n_total: int = 0, k_used: int = 0) -> int:
+        """Bytes of one rank's exchange buffer."""
+        return cls.__new__(cls)._layout(world, k, d, n_total, k_used)
+
+    def _layout(self, world: int, k: int, d: int, n_total: int, k_used: int) -> int:
+        """Sizes and byte offsets of the exchange buffer - flag pad | 2 x M-step block | 2 x record array | 2 x offsets
+        table - set on ``self``; returns the buffer's size in bytes."""
+        lib = _lib.load()
+        self.world = int(world)
+        self.k, self.d, self.n_total, self.k_used = int(k), int(d), int(n_total), int(k_used)
         self.mstep_bytes = _align(lib.scd_peer_mstep_bytes(self.k, self.d))
         self.per = (self.n_total + self.world - 1) // self.world if self.n_total else 0      # rows per rank (dist.shard_bounds)
         self.rec_w = 1 + self.k_used
         self.rec_bytes = _align(self.world * self.per * self.rec_w * 4) if self.n_total else 0
         self.seg_bytes = _align(self.world * (self.k + 1) * 4) if self.n_total else 0      # [world, K + 1] offsets of the sorted runs
-        self.off_mstep = flag_bytes
+        self.off_mstep = _align(lib.scd_peer_flag_bytes())
         self.off_rec = self.off_mstep + 2 * self.mstep_bytes
         self.off_seg = self.off_rec + 2 * self.rec_bytes
-        total = self.off_seg + 2 * self.seg_bytes
-        self.buf = symm_mem.empty(total, dtype=torch.uint8, device=dev)
-        self.buf.zero_()
-        self.handle = symm_mem.rendezvous(self.buf, self.group.group_name)
-        torch.cuda.synchronize(dev)
-        dist.barrier(group=self.group)                      # every pad is zero before anybody signals
-        ptrs = [int(p) for p in self.handle.buffer_ptrs]
+        return self.off_seg + 2 * self.seg_bytes
+
+    def _carve(self, world: int, rank: int, k: int, d: int, n_total: int, k_used: int, buf: torch.Tensor, ptrs):
+        """Lays out this rank's exchange buffer ``buf`` (``buffer_bytes`` long, zeroed) and takes its views; ``ptrs[r]`` is
+        rank r's buffer as this rank addresses it.  Needs no process group: the tests run the exchange kernels on one GPU
+        with ordinary allocations standing in for the ranks' mapped buffers."""
+        if buf.numel() < self._layout(world, k, d, n_total, k_used):
+            raise ValueError('exchange buffer smaller than its layout')
+        self.rank = int(rank)
+        self.buf = buf
         self.table = (C.c_void_p * self.world)(*ptrs)       # rank -> base of its exchange buffer, mapped here
         self._mstep_parity = 0
         self._rec_parity = 0
